@@ -7,6 +7,7 @@ threshold (epsilon) graphs of the same path as a second block of the same JSON l
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
         --master-port 29500 bench.py --gpus 8 --steps 3 --warmup 3
     python bench.py --impl reference --steps 3 --warmup 1      # CPU arm (oracle port)
+    python bench.py --steps 3 --warmup 3 --dump-outputs bench_outputs   # + the last step's kNN lists as .npy
 
 A step = one full graph build: pack the token table into bit planes, build the kNN lists of
 all N rows with the fused Hamming+top-k sweeps, finalise, exchange.  The build is the symmetric
@@ -65,7 +66,15 @@ def parse_args():
     ap.add_argument("--no-queries", action="store_true", help="skip the distance-to-dataset query block (C5)")
     ap.add_argument("--one-sided", action="store_true",
                     help="evaluate all N^2 ordered pairs with the one-sided sweep (no symmetry)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the kNN lists of the last one as DIR/knn_{rows,idx,w}.npy "
+                         "(float64; a fixed, seeded sample of rows on large tables)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU build computed: it needs --impl b200")
+    return args
 
 
 def make_tokens(n, L, kind, seed=0):
@@ -273,6 +282,23 @@ def sample_rows(n, world, eng, words, boot, count=256, seed=7):
     return np.array(sorted(rows), dtype=np.int64)
 
 
+DUMP_BYTES = 32 << 20     # idx + w written by --dump-outputs (the row list adds at most 1/(2k) of that)
+
+
+def dump_knn(out_dir, idx, w):
+    """--dump-outputs: the (idx, w) lists of a kNN build -- what build_neighbours hands its caller -- as
+    float64 .npy files (exact for every index and integer distance).  Tables whose lists exceed
+    DUMP_BYTES are written for a fixed, seeded sample of rows; knn_rows.npy lists the rows written."""
+    import torch
+    n, kk = idx.shape
+    cap = max(1, DUMP_BYTES // (16 * max(1, kk)))
+    rows = np.arange(n) if n <= cap else np.sort(np.random.default_rng(0).choice(n, size=cap, replace=False))
+    sel = torch.from_numpy(rows).to(idx.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("rows", rows), ("idx", idx[sel].cpu().numpy()), ("w", w[sel].cpu().numpy())):
+        np.save(os.path.join(out_dir, f"knn_{name}.npy"), a.astype(np.float64))
+
+
 def all_true(flag, world, device):
     import torch
     import torch.distributed as dist
@@ -372,6 +398,8 @@ def run_b200(args):
     eng.time_sweeps(False)
     launches = eng.launch_count(reset=True)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_knn(args.dump_outputs, *last["knn"])
     pairs = float(n) * float(n)
     value = pairs * args.steps / (ms_total * 1e-3) / 1e9
 

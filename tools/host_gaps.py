@@ -1,5 +1,5 @@
 import os, sys, time, operator
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from bench import make_gb1_library, make_tokens
 from prograph_b200 import graph
