@@ -108,7 +108,10 @@ size_t pg_eps_workspace_bytes_capture(int64_t own_rows, int64_t stream_rows, int
  * For every own row r in [row0,row0+rows): the first (drop+k) stream rows in
  * (distance, index) order; positions [drop, drop+k) are written:
  *   out_idx[r*k + j]  int64,  out_w[r*k + j] per `weight`.
- * If stream_rows < drop+k the tail is filled with idx = -1.  */
+ * If stream_rows < drop+k the tail is filled with idx = -1 and weight 0 (int64 0, or 0.0f for
+ * similarities; the same for every kNN output of this library).  The lists of 256 own rows live in
+ * shared memory: k + drop <= 78, fewer on rows of more than 1024 residues (their ring takes more
+ * room), else PG_ERR_UNSUPPORTED.  */
 int pg_hamming_knn(const uint32_t* own, int64_t own_rows, int64_t row0, int64_t rows,
                    const uint32_t* stream_tab, int64_t stream_rows,
                    int planes, int words, int k, int drop, int weight,
@@ -275,7 +278,10 @@ int pg_minkowski2_gemm_tile(const uint8_t* A, const int32_t* normA, int64_t M,
                             const uint8_t* B, const int32_t* normB, int64_t N, int K,
                             int value_kind, int similarity, void* out, int64_t ld, void* stream);
 /* fused kNN (prograph.py:755-765 with distance=minkowski): sorted positions [drop, drop+k) of every
- * query row in (value, index) order -- descending value for similarity; out_val fp16 / float32 */
+ * query row in (value, index) order -- descending value for similarity; out_val fp16 / float32.
+ * If N < drop+k the tail is filled with idx = -1 and value 0 (as pg_hamming_knn).  The lists of 256
+ * query rows share shared memory with the operand ring: k + drop <= 68 at K = 32, 63 at K = 64, 31 at
+ * K = 256, else PG_ERR_UNSUPPORTED. */
 int pg_minkowski2_gemm_knn(const uint8_t* A, const int32_t* normA, int64_t M,
                            const uint8_t* B, const int32_t* normB, int64_t N, int K,
                            int value_kind, int similarity, int k, int drop,

@@ -458,6 +458,13 @@ __global__ void __launch_bounds__(GTHREADS, 1) mink_gemm_kernel(const __grid_con
             }
           }
         } else {
+          // pad columns of the last B tile (index >= N) are never candidates: their S is huge but
+          // finite, so with fewer than k1 dataset rows they would fill the empty list slots
+          if (col0 + 32 > prm.N) {
+#pragma unroll
+            for (int j = 0; j < 32; ++j)
+              if (col0 + j >= prm.N) v[j] = 0x7fffffff;
+          }
           // tree minimum of the 32 values (a linear chain would serialise 31 dependent mins)
           int m8[8];
 #pragma unroll

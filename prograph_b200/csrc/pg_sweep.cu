@@ -169,8 +169,11 @@ __device__ __forceinline__ void emit_key(unsigned long long best, long long at, 
   if (keys_out) {
     out_keys[at] = best;
   } else if (best == ~0ull) {
+    // missing entry: index -1, weight 0 in every weight kind (0.0, not the similarity of d = 0),
+    // as the Minkowski GEMM writes it
     out_idx[at] = -1;
-    write_weight(out_w, at, 0, weight);
+    if (weight == PG_W_SIM_F32) reinterpret_cast<float*>(out_w)[at] = 0.0f;
+    else write_weight(out_w, at, 0, weight);
   } else {
     out_idx[at] = static_cast<long long>(best & 0xffffffffull);
     write_weight(out_w, at, static_cast<int>(best >> 32), weight);

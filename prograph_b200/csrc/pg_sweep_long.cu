@@ -141,9 +141,12 @@ __global__ void __launch_bounds__(kSweepThreads, 2) sweep_long_kernel(const __gr
         for (int j = 0; j < LBN; ++j) acc[j] += ham_chunk<P>(q, tile + j * COLW + ch * LCH, Wt, one);
       }
       if (ncols < LBN) {      // table end: the zero pad rows must never look like neighbours
+        // kNN: all ones, which fails the candidate test even against the empty threshold of a list
+        // that is not full yet (stream rows < k1); the range and LUT tests reject 0x3fffffff
+        const int pad = MODE == MODE_KNN ? -1 : 0x3fffffff;
 #pragma unroll
         for (int j = 0; j < LBN; ++j)
-          if (j >= ncols) acc[j] = 0x3fffffff;
+          if (j >= ncols) acc[j] = pad;
       }
 
       if constexpr (MODE == MODE_KNN) {
