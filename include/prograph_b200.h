@@ -317,10 +317,14 @@ int pg_tile_topk(const void* tile, int dtype, int64_t rows, int64_t N, int64_t l
 /* threshold test of prograph.py:734-736 / :544 on a tile:
  *   keep = cmp(v, eps)            swap = 0
  *   keep = cmp(eps, v)            swap = 1   (similarity: operands swapped, :734)
- *   and, per `guard`: 0 none, 1  v > 0  (:736),  2  v < 1  (:734).
- * eps is rounded to the tile dtype first (a python scalar is compared in the tensor's
- * dtype).  Pass 1 writes counts[r]; pass 2 writes ascending column indices and the
- * values at indptr[r].. ; `tile` may also be a uint8 mask (dtype PG_U8, cmp ignored). */
+ *   and, per `guard & 3`: 0 none, 1  v > 0  (:736),  2  v < 1  (:734).
+ * eps is compared the way torch compares a tensor with a python scalar: for fp16 / float32 /
+ * float64 tiles it is rounded to the tile dtype; for int32 / int64 tiles it is compared exactly
+ * (a python int, |v| <= 2^53), unless `guard` carries PG_EPS_FLOAT (a python float): then both
+ * operands are rounded to float32 and compared there, as torch promotes int < float to float32.
+ * Pass 1 writes counts[r]; pass 2 writes ascending column indices and the values at
+ * indptr[r].. ; `tile` may also be a uint8 mask (dtype PG_U8, cmp ignored). */
+#define PG_EPS_FLOAT 4
 int pg_tile_threshold_count(const void* tile, int dtype, int64_t rows, int64_t N, int64_t ld,
                             int cmp, double eps, int swap, int guard, int64_t* counts, void* stream);
 int pg_tile_threshold_fill(const void* tile, int dtype, int64_t rows, int64_t N, int64_t ld,

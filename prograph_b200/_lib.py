@@ -18,6 +18,8 @@ U8, I16, I32, I64, F16, F32, F64 = range(7)
 LT, LE, EQ, NE, GE, GT = range(6)
 # pgWeight
 W_I64, W_SIM_F32, W_I32, W_FLAG_U8 = range(4)
+# flag bit of the threshold kernels' `guard`: eps is a python float (PG_EPS_FLOAT)
+EPS_FLOAT = 4
 
 
 class Unsupported(RuntimeError):

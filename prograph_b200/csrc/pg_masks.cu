@@ -7,11 +7,13 @@
 #include <cub/device/device_select.cuh>
 #include <thrust/iterator/counting_iterator.h>
 
+#include <vector>
+
 #include "pg_common.cuh"
 
 namespace pg {
 
-constexpr int kMaxMaskWords = 128;  // sequences up to 4096 residues for the selection kernels
+constexpr int kMaxMaskWords = 128;  // selection masks passed as kernel parameters: rows up to 4096 residues
 
 struct WordVec { uint32_t w[kMaxMaskWords]; };
 struct LutVec { uint32_t w[kMaxMaskWords + 1]; };     // truth table over d = 0 .. 32*words: one word more
@@ -98,23 +100,40 @@ __global__ void mutant_any_kernel(const uint32_t* __restrict__ mut, long long N,
   }
 }
 
-__global__ void select_rows_kernel(const uint32_t* __restrict__ mut, long long N, int words, LutVec dist_lut,
-                                   int use_lut, WordVec inside, WordVec outside, int pos_mode,
-                                   uint8_t* __restrict__ flag) {
+// The masks of the selection: rows of up to kMaxMaskWords words take them as kernel parameters
+// (constant-bank reads, nothing to copy); longer rows read them from a small device buffer.
+struct ParamMasks {
+  LutVec lut;
+  WordVec inside, outside;
+  __device__ uint32_t in(int w) const { return inside.w[w]; }
+  __device__ uint32_t out(int w) const { return outside.w[w]; }
+  __device__ uint32_t lut_word(int i) const { return lut.w[i]; }
+};
+struct BufferMasks {
+  const uint32_t* buf;   // [inside: words][outside: words][lut: words + 1]
+  int words;
+  __device__ uint32_t in(int w) const { return __ldg(buf + w); }
+  __device__ uint32_t out(int w) const { return __ldg(buf + words + w); }
+  __device__ uint32_t lut_word(int i) const { return __ldg(buf + 2 * words + i); }
+};
+
+template <typename Masks>
+__global__ void select_rows_kernel(const uint32_t* __restrict__ mut, long long N, int words, const Masks masks,
+                                   int use_lut, int pos_mode, uint8_t* __restrict__ flag) {
   for (long long n = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; n < N;
        n += static_cast<long long>(gridDim.x) * blockDim.x) {
     const uint32_t* m = mut + static_cast<size_t>(n) * words;
     int d = 0;
     bool any_in = false, all_in = true, none_out = true;
     for (int w = 0; w < words; ++w) {
-      const uint32_t v = m[w], in = inside.w[w];
+      const uint32_t v = m[w], in = masks.in(w);
       d += __popc(v);
       any_in |= (v & in) != 0;
       all_in &= (v & in) == in;
-      none_out &= (v & outside.w[w]) == 0;
+      none_out &= (v & masks.out(w)) == 0;
     }
     bool ok = true;
-    if (use_lut) ok = (dist_lut.w[d >> 5] >> (d & 31)) & 1u;
+    if (use_lut) ok = (masks.lut_word(d >> 5) >> (d & 31)) & 1u;
     if (pos_mode == 1) ok = ok && any_in && none_out;
     else if (pos_mode == 2) ok = ok && all_in && none_out;
     else if (pos_mode == 3) ok = ok && !any_in;
@@ -331,24 +350,40 @@ int pg_compact_columns(const uint32_t* table, int64_t N, int planes, int words, 
 int pg_select_rows(const uint32_t* mut, int64_t N, int words, const uint32_t* dist_lut_host, int lut_words,
                    const uint32_t* inside_host, const uint32_t* outside_host, int pos_mode, uint8_t* flag,
                    void* stream) {
-  PG_CHECK_ARG(mut && flag && N > 0, "bad arguments");
-  PG_CHECK_ARG(words > 0 && words <= kMaxMaskWords, "selection kernels support up to %d words", kMaxMaskWords);
+  PG_CHECK_ARG(mut && flag && N > 0 && words > 0, "bad arguments");
   PG_CHECK_ARG(pos_mode >= 0 && pos_mode <= 3, "bad pos_mode %d", pos_mode);
   PG_CHECK_ARG(pos_mode == 0 || inside_host, "positions mask missing");
-  PG_CHECK_ARG(!dist_lut_host || (lut_words >= 1 && lut_words <= kMaxMaskWords + 1 && lut_words * 32 > words * 32),
+  PG_CHECK_ARG(!dist_lut_host || (lut_words >= 1 && lut_words <= words + 1 && lut_words * 32 > words * 32),
                "distance lut must cover 0..%d", words * 32);
   PG_CHECK_ARG(!(pos_mode == 1 || pos_mode == 2) || outside_host, "unchanged-positions mask missing");
-  LutVec lut;
-  WordVec inside, outside;
-  memset(&lut, 0, sizeof(lut));
-  memset(&inside, 0, sizeof(inside));
-  memset(&outside, 0, sizeof(outside));
-  if (outside_host) memcpy(outside.w, outside_host, sizeof(uint32_t) * words);
-  if (dist_lut_host) memcpy(lut.w, dist_lut_host, sizeof(uint32_t) * lut_words);
-  if (inside_host) memcpy(inside.w, inside_host, sizeof(uint32_t) * words);
-  select_rows_kernel<<<grid_for(N, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      mut, N, words, lut, dist_lut_host ? 1 : 0, inside, outside, pos_mode, flag);
-  PG_LAUNCH_CHECK();
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int use_lut = dist_lut_host ? 1 : 0;
+  if (words <= kMaxMaskWords) {
+    ParamMasks m;
+    memset(&m, 0, sizeof(m));
+    if (outside_host) memcpy(m.outside.w, outside_host, sizeof(uint32_t) * words);
+    if (dist_lut_host) memcpy(m.lut.w, dist_lut_host, sizeof(uint32_t) * lut_words);
+    if (inside_host) memcpy(m.inside.w, inside_host, sizeof(uint32_t) * words);
+    select_rows_kernel<ParamMasks><<<grid_for(N, 256), 256, 0, s>>>(mut, N, words, m, use_lut, pos_mode, flag);
+    PG_LAUNCH_CHECK();
+    return PG_OK;
+  }
+  // rows longer than 32 * kMaxMaskWords residues: the masks go through a device buffer
+  std::vector<uint32_t> host(static_cast<size_t>(3 * words + 1), 0u);
+  if (inside_host) memcpy(host.data(), inside_host, sizeof(uint32_t) * words);
+  if (outside_host) memcpy(host.data() + words, outside_host, sizeof(uint32_t) * words);
+  if (dist_lut_host) memcpy(host.data() + 2 * words, dist_lut_host, sizeof(uint32_t) * lut_words);
+  void* buf = nullptr;
+  PG_CUDA(temp_alloc(&buf, sizeof(uint32_t) * host.size(), s));
+  cudaError_t e = cudaMemcpyAsync(buf, host.data(), sizeof(uint32_t) * host.size(), cudaMemcpyHostToDevice, s);
+  if (e == cudaSuccess) {
+    BufferMasks m{static_cast<const uint32_t*>(buf), words};
+    select_rows_kernel<BufferMasks><<<grid_for(N, 256), 256, 0, s>>>(mut, N, words, m, use_lut, pos_mode, flag);
+    count_launch();
+    e = cudaGetLastError();
+  }
+  cudaFreeAsync(buf, s);
+  if (e != cudaSuccess) { set_error("select rows failed: %s", cudaGetErrorString(e)); return PG_ERR_CUDA; }
   return PG_OK;
 }
 

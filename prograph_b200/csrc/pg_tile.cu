@@ -237,22 +237,40 @@ __global__ void __launch_bounds__(256) elem_tile_kernel(const ElemParams prm) {
   }
 }
 
+// bytes of one output entry of elem_tile_kernel
+template <typename T, int VK, int METRIC>
+static size_t elem_out_bytes(const ElemParams& prm) {
+  if (METRIC == 1) return prm.weight == PG_W_I64 ? 8 : 4;
+  if (VK == VK_F16) return 2;
+  if (VK == VK_F64) return 8;
+  return 4;                                       // float32 out for f32 and int64 inputs
+}
+
 template <typename T, int VK, int METRIC>
 static int launch_elem(const ElemParams& prm, int pk_in, int pk_root, cudaStream_t s) {
-  dim3 grid(static_cast<unsigned>(ceil_div(prm.N, ET_N)), static_cast<unsigned>(ceil_div(prm.qrows, ET_M)));
-#define PG_EL(PI, PR) elem_tile_kernel<T, VK, METRIC, PI, PR><<<grid, 256, 0, s>>>(prm)
-  if (METRIC == 1) {
-    PG_EL(PK_ONE, PK_ONE);
-  } else {
-    // the common pairs get their own instantiation; everything else takes the powf path
-    if (pk_in == PK_TWO && pk_root == PK_SQRT) PG_EL(PK_TWO, PK_SQRT);
-    else if (pk_in == PK_ONE && pk_root == PK_ONE) PG_EL(PK_ONE, PK_ONE);
-    else if (pk_in == PK_THREE) PG_EL(PK_THREE, PK_GENERAL);
-    else if (pk_in == PK_SQRT && pk_root == PK_TWO) PG_EL(PK_SQRT, PK_TWO);
-    else PG_EL(PK_GENERAL, PK_GENERAL);
-  }
+  // query blocks go on gridDim.y (at most 65535): larger tiles are launched in chunks of query rows
+  constexpr long long kChunk = 65535ll * ET_M;
+  const size_t row_bytes = static_cast<size_t>(prm.ld) * elem_out_bytes<T, VK, METRIC>(prm);
+  for (long long c0 = 0; c0 < prm.qrows; c0 += kChunk) {
+    ElemParams part = prm;
+    part.q0 = prm.q0 + c0;
+    part.qrows = std::min(kChunk, prm.qrows - c0);
+    part.out = static_cast<char*>(prm.out) + static_cast<size_t>(c0) * row_bytes;
+    dim3 grid(static_cast<unsigned>(ceil_div(part.N, ET_N)), static_cast<unsigned>(ceil_div(part.qrows, ET_M)));
+#define PG_EL(PI, PR) elem_tile_kernel<T, VK, METRIC, PI, PR><<<grid, 256, 0, s>>>(part)
+    if (METRIC == 1) {
+      PG_EL(PK_ONE, PK_ONE);
+    } else {
+      // the common pairs get their own instantiation; everything else takes the powf path
+      if (pk_in == PK_TWO && pk_root == PK_SQRT) PG_EL(PK_TWO, PK_SQRT);
+      else if (pk_in == PK_ONE && pk_root == PK_ONE) PG_EL(PK_ONE, PK_ONE);
+      else if (pk_in == PK_THREE) PG_EL(PK_THREE, PK_GENERAL);
+      else if (pk_in == PK_SQRT && pk_root == PK_TWO) PG_EL(PK_SQRT, PK_TWO);
+      else PG_EL(PK_GENERAL, PK_GENERAL);
+    }
 #undef PG_EL
-  PG_LAUNCH_CHECK();
+    PG_LAUNCH_CHECK();
+  }
   return PG_OK;
 }
 
@@ -600,8 +618,7 @@ struct ThreshParams {
   int cmp, swap, guard;
   float eps_f;
   double eps_d;
-  long long eps_i;
-  int eps_is_int;
+  int eps_is_int;     // integer tiles: compare exactly (python int eps) instead of in float32
 };
 
 __device__ __forceinline__ bool cmp_apply(int cmp, double a, double b) {
@@ -615,7 +632,9 @@ __device__ __forceinline__ bool cmp_apply(int cmp, double a, double b) {
   }
 }
 // v is converted exactly to double for every supported dtype except |int64| > 2^53 (not a
-// distance).  eps was rounded to the tile dtype on the host (fp16 / fp32) as torch does.
+// distance).  eps was rounded to the tile dtype on the host (fp16 / fp32) as torch does.  An
+// integer tile against a python float compares in float32 (torch's promotion): both operands are
+// rounded to float32, whose values double holds exactly.
 template <typename T> __device__ __forceinline__ double as_double(T v) { return static_cast<double>(v); }
 template <> __device__ __forceinline__ double as_double<__half>(__half v) { return static_cast<double>(__half2float(v)); }
 
@@ -623,7 +642,8 @@ template <typename T>
 __device__ __forceinline__ bool keep_value(T v, const ThreshParams& tp) {
   if (sizeof(T) == 1) return v != T(0);  // mask input
   const double x = as_double<T>(v);
-  const bool c = tp.swap ? cmp_apply(tp.cmp, tp.eps_d, x) : cmp_apply(tp.cmp, x, tp.eps_d);
+  const double xc = (std::is_integral<T>::value && !tp.eps_is_int) ? static_cast<double>(static_cast<float>(v)) : x;
+  const bool c = tp.swap ? cmp_apply(tp.cmp, tp.eps_d, xc) : cmp_apply(tp.cmp, xc, tp.eps_d);
   if (tp.guard == 1) return c && (x > 0.0);
   if (tp.guard == 2) return c && (x < 1.0);
   return c;
@@ -687,17 +707,19 @@ __global__ void __launch_bounds__(256) tile_thresh_fill_kernel(const T* __restri
 
 static int fill_thresh(ThreshParams& tp, int dtype, int cmp, double eps, int swap, int guard) {
   PG_CHECK_ARG(cmp >= PG_LT && cmp <= PG_GT, "bad comparison opcode %d", cmp);
-  PG_CHECK_ARG(guard >= 0 && guard <= 2, "bad guard %d", guard);
+  const int kind = guard & ~PG_EPS_FLOAT;
+  PG_CHECK_ARG(kind >= 0 && kind <= 2, "bad guard %d", guard);
   tp.cmp = cmp;
   tp.swap = swap;
-  tp.guard = guard;
-  // a python scalar is compared in the tensor's dtype: round eps the way torch does
+  tp.guard = kind;
+  // a python scalar is compared the way torch compares it: rounded to a float tile's dtype; exactly
+  // against an integer tile when it is an int; in float32 against an integer tile when it is a float
+  tp.eps_is_int = (guard & PG_EPS_FLOAT) ? 0 : 1;
+  const bool to_f32 = dtype == PG_F32 || ((dtype == PG_I32 || dtype == PG_I64) && !tp.eps_is_int);
   if (dtype == PG_F16) tp.eps_d = static_cast<double>(__half2float(__float2half_rn(static_cast<float>(eps))));
-  else if (dtype == PG_F32) tp.eps_d = static_cast<double>(static_cast<float>(eps));
+  else if (to_f32) tp.eps_d = static_cast<double>(static_cast<float>(eps));
   else tp.eps_d = eps;
   tp.eps_f = static_cast<float>(tp.eps_d);
-  tp.eps_i = static_cast<long long>(eps);
-  tp.eps_is_int = 0;
   return PG_OK;
 }
 

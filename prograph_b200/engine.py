@@ -2,6 +2,7 @@
 is a C-ABI call into libprograph_b200.so (hand-written sm_100a kernels).  No CPU fallback anywhere.
 """
 import ctypes as C
+import numbers
 
 import numpy as np
 import torch
@@ -500,21 +501,29 @@ class CudaEngine:
                                       1 if descending else 0, _ptr(idx), _ptr(val), self._stream()))
         return idx, val
 
+    @staticmethod
+    def _thresh_guard(eps, guard):
+        """`guard` with L.EPS_FLOAT set when eps is a python float: torch compares an integer tile
+        with an int exactly and with a float in float32 (pg_tile_threshold_count)."""
+        return int(guard) | (0 if isinstance(eps, numbers.Integral) else L.EPS_FLOAT)
+
     def tile_threshold_counts(self, tile, cmp, eps, swap=False, guard=0):
         """Per-row number of tile entries passing the threshold test (pg_tile_threshold_count)."""
         rows, N = tile.shape
         counts = self.empty((rows,), torch.int64)
         L.check(self.lib.pg_tile_threshold_count(_ptr(tile), _PG_DTYPE[tile.dtype], rows, N, int(tile.stride(0)), int(cmp),
-                                                 float(eps), 1 if swap else 0, int(guard), _ptr(counts), self._stream()))
+                                                 float(eps), 1 if swap else 0, self._thresh_guard(eps, guard), _ptr(counts),
+                                                 self._stream()))
         return counts
 
     def tile_threshold(self, tile, cmp, eps, swap=False, guard=0, values=True):
         """CSR of the tile entries passing the threshold test (see pg_tile_threshold_count)."""
         rows, N = tile.shape
         dt = _PG_DTYPE[tile.dtype]
+        guard = self._thresh_guard(eps, guard)
         counts = self.empty((rows,), torch.int64)
         L.check(self.lib.pg_tile_threshold_count(_ptr(tile), dt, rows, N, int(tile.stride(0)), int(cmp), float(eps),
-                                                 1 if swap else 0, int(guard), _ptr(counts), self._stream()))
+                                                 1 if swap else 0, guard, _ptr(counts), self._stream()))
         indptr = self.exclusive_scan(counts)
         nnz = int(indptr[-1].item())
         self.check_edge_budget(nnz)
@@ -522,7 +531,7 @@ class CudaEngine:
         val = self.empty((nnz,), tile.dtype) if values else None
         if nnz:
             L.check(self.lib.pg_tile_threshold_fill(_ptr(tile), dt, rows, N, int(tile.stride(0)), int(cmp), float(eps),
-                                                    1 if swap else 0, int(guard), _ptr(indptr), _ptr(idx), _ptr(val),
+                                                    1 if swap else 0, guard, _ptr(indptr), _ptr(idx), _ptr(val),
                                                     self._stream()))
         return indptr, idx, val
 
