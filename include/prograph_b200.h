@@ -266,6 +266,11 @@ int pg_hamming_values_tile(const void* X, int64_t N, const void* Y, int64_t M, i
  * Operand tables: uint8 rows in K-major 8x16-byte core-matrix order
  *   byte(r, k) = ((r/8)*(K/16) + k/16)*128 + (r%8)*16 + k%16,  K = pg_gemm_width(L),
  * padded to pg_gemm_rows(N) rows, plus int32 squared norms per row (pad rows: 0x3fffffff).
+ * K <= 8192 (PG_ERR_UNSUPPORTED above): up to K = 256 the two A tiles of a CTA stay resident in
+ * shared memory, wider rows stream 128-wide K-chunks of both A tiles and the B tile through the ring
+ * (same layout, same results).  With tokens <= 255, S <= 255^2 * 8192 stays below 2^29.
+ * Measured on one B200 at a 1000 W power limit, kNN k=1 over 262 144 rows: 685 / 283 / 69 Gpairs/s at
+ * K = 512 / 1184 / 5376, L2-bound (profiles/gemm_wide_time.log).
  * ------------------------------------------------------------------------- */
 int     pg_gemm_width(int L);
 int64_t pg_gemm_rows(int64_t N);
@@ -281,7 +286,7 @@ int pg_minkowski2_gemm_tile(const uint8_t* A, const int32_t* normA, int64_t M,
  * query row in (value, index) order -- descending value for similarity; out_val fp16 / float32.
  * If N < drop+k the tail is filled with idx = -1 and value 0 (as pg_hamming_knn).  The lists of 256
  * query rows share shared memory with the operand ring: k + drop <= 68 at K = 32, 63 at K = 64, 31 at
- * K = 256, else PG_ERR_UNSUPPORTED. */
+ * K = 256, 42 at every K in (256, 8192] (K-chunked ring), else PG_ERR_UNSUPPORTED. */
 int pg_minkowski2_gemm_knn(const uint8_t* A, const int32_t* normA, int64_t M,
                            const uint8_t* B, const int32_t* normB, int64_t N, int K,
                            int value_kind, int similarity, int k, int drop,

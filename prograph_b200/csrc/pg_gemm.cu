@@ -26,7 +26,10 @@
 //   * epilogues: materialised tile (minkowski.py:36-40) or fused kNN: a candidate test in
 //     S-space against a per-row integer threshold (min + one vote per 32 columns), rare
 //     warp-cooperative insertion into a sorted (value, index) list in shared memory; the
-//     N x N matrix never reaches HBM.
+//     N x N matrix never reaches HBM;
+//   * rows wider than GMAX_RESIDENT_K (CHUNKED): the A tiles no longer fit, so every ring stage
+//     carries one GKC-wide K-chunk of A tile 0, A tile 1 and the B tile, and the issuers accumulate
+//     the chunks of a B tile into the same TMEM accumulator; the epilogues are unchanged.
 #include <cstdlib>
 
 #include "pg_sweep.cuh"   // knn_insert_coop, kMaxListRounds
@@ -45,6 +48,15 @@ constexpr int GPROD_LANES = 8;  // lanes of the producer warp that each copy a s
 constexpr int GACC = 4;         // TMEM accumulators (4 x 128 columns = all 512): two per A tile
 constexpr int GNORM_SLOTS = 8;  // ring of per-tile dataset norms (512 B each)
 constexpr int PAD_NORM = 0x3fffffff;
+constexpr int GMAX_RESIDENT_K = 256;   // widest row whose two A tiles stay resident next to the B ring
+constexpr int GKC = 128;        // K-chunk of the chunked mode: a stage is 3 x 16 KB, so three stages fit next to
+                                // the tile-store staging and two next to 42-entry lists (256 would leave one / ten)
+// Widest row (K) of the GEMM.  With tokens <= 255, S <= 255^2 * 8192 = 532 684 800 < PAD_NORM / 2 =
+// 536 870 911, the bound gemm_eps_common enforces on the S range, and a pad column's S = nq + PAD_NORM
+// stays below 2^31, so every sum of the epilogues is exact in int32.  With the fp16 chain's tokens
+// <= 31, S <= 961 * 8192 < 2^24: torch's fp32 accumulation of the fp16 squares is exact and the
+// reference's value is still fp16(sqrt(fp16(S))).
+constexpr int GMAX_K = 8192;
 
 enum GemmValue { GV_F16 = 0, GV_F32 = 1 };     // which rounding chain turns S into the distance
 enum GemmMode { GM_TILE = 0, GM_KNN = 1, GM_COUNT = 2, GM_FILL = 3 };
@@ -202,7 +214,7 @@ __device__ __forceinline__ void mbar_wait_poll(uint64_t* bar, uint32_t parity) {
     if (++spins > (1u << 26)) __trap();
   }
 }
-template <int VK, int MODE, int ISSUERS>
+template <int VK, int MODE, int ISSUERS, bool CHUNKED>
 __global__ void __launch_bounds__(GTHREADS, 1) mink_gemm_kernel(const __grid_constant__ GemmParams prm) {
   extern __shared__ __align__(1024) unsigned char smem[];
   const int K = prm.K;
@@ -210,7 +222,9 @@ __global__ void __launch_bounds__(GTHREADS, 1) mink_gemm_kernel(const __grid_con
   uint8_t* sA = smem;                                     // [GA] tiles
   uint8_t* sB = smem + GA * tile_bytes;
   const int n_stages = prm.stages;
-  int* sNorm = reinterpret_cast<int*>(smem + tile_bytes * (GA + n_stages));       // [GNORM_SLOTS][GN]
+  // CHUNKED: the ring is [stages][A tile 0, A tile 1, B tile][GM rows x GKC] and nothing is resident
+  constexpr uint32_t chunk_bytes = GM * GKC;
+  int* sNorm = reinterpret_cast<int*>(smem + (CHUNKED ? 3 * chunk_bytes * n_stages : tile_bytes * (GA + n_stages)));   // [GNORM_SLOTS][GN]
   uint64_t* bars = reinterpret_cast<uint64_t*>(sNorm + GNORM_SLOTS * GN);
   uint64_t* full = bars;                  // [GSTAGES] B tile (+ its norms) landed
   uint64_t* empty = bars + GSTAGES;       // [GSTAGES] MMAs reading the stage have completed
@@ -254,6 +268,38 @@ __global__ void __launch_bounds__(GTHREADS, 1) mink_gemm_kernel(const __grid_con
     // GPROD_LANES lanes each issue a slice of the tile so that several bulk requests are in flight
     // (measured neutral against one 32 KB request; the kernel is not copy-bound, see
     // profiles/r1_ncu_notes.md).
+    if constexpr (CHUNKED) {
+      // In the global table the K-chunk [c0, c0 + kc) of an 8-row group is kc * 8 contiguous bytes at
+      // (row / 8) * 8K + c0 * 8, and in the ring it sits at SBO = GKC * 8 intervals (a narrower last
+      // chunk leaves the end of each interval unused): lane g < 16 copies row group g of all three tiles.
+      const int nchunks = (K + GKC - 1) / GKC;
+      int stage = 0;
+      uint32_t phase = 0;
+      for (int t = 0; t < n_tiles; ++t) {
+        for (int c = 0; c < nchunks; ++c) {
+          const int c0 = c * GKC;
+          const uint32_t piece = static_cast<uint32_t>(min(GKC, K - c0)) * 8u;
+          if (lane == 0) {
+            mbar_wait_poll(&empty[stage], phase ^ 1u);
+            mbar_arrive_expect_tx(&full[stage], 3 * (GM / 8) * piece + (c == 0 ? GN * 4 : 0));
+            // norms ride with the first chunk; slot reuse (tile t + 8) waits for a stage whose MMAs
+            // (tile >= t + 6: at least two chunks per tile, at most four stages) follow the epilogues of tile t + 4
+            if (c == 0)
+              bulk_g2s(sNorm + (t % GNORM_SLOTS) * GN, prm.normB + static_cast<size_t>(t_begin + t) * GN, GN * 4,
+                       &full[stage]);
+          }
+          __syncwarp();
+          if (lane < GM / 8) {
+            uint8_t* dst = smem + static_cast<size_t>(stage) * 3 * chunk_bytes + lane * (GKC * 8);
+            const size_t off = static_cast<size_t>(lane) * 8 * K + static_cast<size_t>(c0) * 8;
+            bulk_g2s(dst, prm.A + static_cast<size_t>(row0) * K + off, piece, &full[stage]);
+            bulk_g2s(dst + chunk_bytes, prm.A + static_cast<size_t>(row0 + GM) * K + off, piece, &full[stage]);
+            bulk_g2s(dst + 2 * chunk_bytes, prm.B + static_cast<size_t>(t_begin + t) * GN * K + off, piece, &full[stage]);
+          }
+          if (++stage == n_stages) { stage = 0; phase ^= 1u; }
+        }
+      }
+    } else {
     if (lane == 0) {        // both A tiles: 256 consecutive rows of the core-matrix table (padded to GROWS)
       mbar_arrive_expect_tx(a_full, GA * tile_bytes);
       bulk_g2s(sA, prm.A + static_cast<size_t>(row0) * K, tile_bytes, a_full);
@@ -280,6 +326,7 @@ __global__ void __launch_bounds__(GTHREADS, 1) mink_gemm_kernel(const __grid_con
       }
       if (++stage == n_stages) { stage = 0; phase ^= 1u; }
     }
+    }
   } else if (warp >= GMMA_WARP) {
     // ---------------- MMA issuers ----------------
     // issuers == 2: warp GMMA_WARP + a multiplies A tile a with every B tile (short lists / queries: the
@@ -289,6 +336,42 @@ __global__ void __launch_bounds__(GTHREADS, 1) mink_gemm_kernel(const __grid_con
     if (lane == 0 && a_first < ISSUERS) {
       // instruction descriptor: D=S32, A=B=UINT8, K-major both, N=128, M=128
       const uint32_t idesc = (2u << 4) | (static_cast<uint32_t>(GN >> 3) << 17) | (static_cast<uint32_t>(GM >> 4) << 24);
+      if constexpr (CHUNKED) {
+        // The chunks of a B tile accumulate into one accumulator (the flag is 0 only for the first
+        // k-step of the first chunk); every chunk frees its stage, the last one hands the accumulator
+        // to the epilogue.  One descriptor per ring, advanced by 16 units per k-step, chunk_bytes per
+        // operand and 3 * chunk_bytes per stage.
+        constexpr uint32_t chunk_units = chunk_bytes >> 4;
+        const uint64_t desc0 = umma_desc(smem_u32(smem), 128, GKC * 8);
+        const int nchunks = (K + GKC - 1) / GKC;
+        int stage = 0;
+        uint32_t phase = 0;
+        for (int t = 0; t < n_tiles; ++t) {
+          for (int c = 0; c < nchunks; ++c) {
+            const int ksteps = min(GKC, K - c * GKC) / 32;
+            mbar_wait_poll(&full[stage], phase);
+            const uint64_t sdesc = desc0 + static_cast<uint64_t>(stage) * 3 * chunk_units;
+            const uint64_t bdesc = sdesc + 2 * chunk_units;
+#pragma unroll
+            for (int i = 0; i < (ISSUERS == 1 ? GA : 1); ++i) {
+              const int a = ISSUERS == 1 ? i : a_first;
+              const int acc = a + GA * (t & 1);
+              if (c == 0) {
+                mbar_wait_poll(&acc_empty[acc], ((t >> 1) & 1) ^ 1u);
+                tc_fence_after();
+              }
+              const uint64_t adesc = sdesc + static_cast<uint64_t>(a) * chunk_units;
+              const uint32_t d_addr = tmem_base + acc * GN;
+#pragma unroll
+              for (int j = 0; j < GKC / 32; ++j)
+                if (j < ksteps) umma_i8(d_addr, adesc + 16u * j, bdesc + 16u * j, idesc, (c | j) != 0 ? 1u : 0u);
+              if (c == nchunks - 1) umma_commit(&acc_full[acc]);
+            }
+            umma_commit(&empty[stage]);
+            if (++stage == n_stages) { stage = 0; phase ^= 1u; }
+          }
+        }
+      } else {
       const uint32_t sbo = static_cast<uint32_t>(K / 16) * 128u;
       mbar_wait_poll(a_full, 0);
       // Descriptors are built ONCE: a k-step advances the start address by 256 bytes (16 descriptor
@@ -336,6 +419,7 @@ __global__ void __launch_bounds__(GTHREADS, 1) mink_gemm_kernel(const __grid_con
           umma_commit(&empty[stage]);       // the stage may be refilled once BOTH issuers' MMAs have read it
           if (++stage == n_stages) { stage = 0; phase ^= 1u; }
         }
+      }
       }
     }
   } else {
@@ -580,12 +664,12 @@ __global__ void gemm_pack_kernel<__half>(const __half* __restrict__ tokens, long
   }
 }
 
-static size_t gemm_smem_bytes(int K, int k1, int stages, bool tile_mode = false) {
-  return static_cast<size_t>(GM) * K * (GA + stages) + GNORM_SLOTS * GN * 4 + (2 * GSTAGES + 2 * GACC + 1) * sizeof(uint64_t) +
+static size_t gemm_smem_bytes(int K, int k1, int stages, bool tile_mode = false, bool chunked = false) {
+  return (chunked ? static_cast<size_t>(3) * GM * GKC * stages : static_cast<size_t>(GM) * K * (GA + stages)) + GNORM_SLOTS * GN * 4 + (2 * GSTAGES + 2 * GACC + 1) * sizeof(uint64_t) +
          16 + static_cast<size_t>(GROWS) * k1 * 12 + (tile_mode ? 16 + 8 * 32 * 36 * 4 : 0);
 }
 
-template <int VK, int MODE, int ISSUERS>
+template <int VK, int MODE, int ISSUERS, bool CHUNKED>
 static int launch_gemm_issuers(GemmParams prm, cudaStream_t s);
 
 // One MMA-issuing warp (both A tiles, 320 threads) or two (one per A tile, 352 threads).  Two issuers
@@ -596,18 +680,20 @@ template <int VK, int MODE>
 static int launch_gemm(GemmParams prm, cudaStream_t s) {
   int issuers = (MODE == GM_KNN && prm.k1 <= 4) ? 2 : 1;
   if (const char* ev = std::getenv("PG_GEMM_ISSUERS")) issuers = std::atoi(ev) == 2 ? 2 : 1;
-  return issuers == 2 ? launch_gemm_issuers<VK, MODE, 2>(prm, s) : launch_gemm_issuers<VK, MODE, 1>(prm, s);
+  if (prm.K > GMAX_RESIDENT_K)
+    return issuers == 2 ? launch_gemm_issuers<VK, MODE, 2, true>(prm, s) : launch_gemm_issuers<VK, MODE, 1, true>(prm, s);
+  return issuers == 2 ? launch_gemm_issuers<VK, MODE, 2, false>(prm, s) : launch_gemm_issuers<VK, MODE, 1, false>(prm, s);
 }
 
-template <int VK, int MODE, int ISSUERS>
+template <int VK, int MODE, int ISSUERS, bool CHUNKED>
 static int launch_gemm_issuers(GemmParams prm, cudaStream_t s) {
-  auto kern = mink_gemm_kernel<VK, MODE, ISSUERS>;
+  auto kern = mink_gemm_kernel<VK, MODE, ISSUERS, CHUNKED>;
   if (const char* ev = std::getenv("PG_GEMM_DEBUG")) prm.debug = std::atoi(ev);
   prm.issuers = ISSUERS;
   // wide rows / long lists: give up ring stages (down to 2) before giving up the fused path
   size_t smem = 0;
   for (prm.stages = GSTAGES; prm.stages >= 2; --prm.stages) {
-    smem = gemm_smem_bytes(prm.K, MODE == GM_KNN ? prm.k1 : 0, prm.stages, MODE == GM_TILE);
+    smem = gemm_smem_bytes(prm.K, MODE == GM_KNN ? prm.k1 : 0, prm.stages, MODE == GM_TILE, CHUNKED);
     if (smem <= 227 * 1024) break;
   }
   if (smem > 227 * 1024) { set_error("minkowski GEMM: k or row width too large for shared memory (%zu bytes)", smem); return PG_ERR_UNSUPPORTED; }
@@ -748,8 +834,8 @@ static int gemm_common(GemmParams& prm, const uint8_t* A, const int32_t* normA, 
   PG_CHECK_ARG(A && normA && B && normB, "null operand");
   PG_CHECK_ARG(M > 0 && N > 0 && N < (1ll << 32), "bad operand sizes");
   PG_CHECK_ARG(value_kind == GV_F16 || value_kind == GV_F32, "bad value kind %d", value_kind);
-  if (K % 32 != 0 || K < 32 || K > 256) {
-    set_error("minkowski GEMM supports rows of up to 256 tokens (K=%d)", K);
+  if (K % 32 != 0 || K < 32 || K > GMAX_K) {
+    set_error("minkowski GEMM supports rows of up to %d tokens (K=%d)", GMAX_K, K);
     return PG_ERR_UNSUPPORTED;
   }
   memset(&prm, 0, sizeof(prm));

@@ -1,4 +1,6 @@
 """Minkowski distance, drop-in for prograph/distance/minkowski.py:8-41."""
+import math
+
 import torch
 
 from ..engine import get_engine
@@ -17,21 +19,25 @@ def staged_dtype(X, Y, p):
     return torch.float32
 
 
-def gemm_value_kind(dt):
-    """Rounding chain of the tensor-core path for a compute dtype: 0 = fp16 chain (needs tokens
-    <= 31 so that every squared difference is an exact fp16 integer), 1 = float32 root of the
-    exact integer sum (int64 and float32 inputs), None = not applicable."""
+def gemm_value_kind(dt, width=0):
+    """Rounding chain of the tensor-core path for a compute dtype and row width: 0 = fp16 chain
+    (needs tokens <= 31 so that every squared difference is an exact fp16 integer), 1 = float32
+    root of the exact integer sum (int64 and float32 inputs), None = not applicable.  float32 rows
+    are summed in float32, which equals the exact sum only while it stays <= 2^24: their largest
+    token is capped so that width * max_token^2 <= 2^24 (255 up to 258 columns, 45 at 8192)."""
     if dt == torch.float16:
         return 0, 31
-    if dt in (torch.int64, torch.float32):
+    if dt == torch.int64:
         return 1, 255
+    if dt == torch.float32:
+        return 1, min(255, math.isqrt((1 << 24) // max(1, int(width))))
     return None, None
 
 
 def minkowski_matrix(eng, X, Y, p=2, similarity=False):
     from .. import _lib as L
     dt = staged_dtype(X, Y, p)
-    kind, max_token = gemm_value_kind(dt)
+    kind, max_token = gemm_value_kind(dt, X.shape[1])
     if float(p) == 2.0 and kind is not None and X.shape[1] <= eng.GEMM_MAX_WIDTH:
         # p=2 on integer-valued rows is an exact int8 contraction: tensor cores (pg_gemm.cu)
         try:

@@ -425,7 +425,8 @@ class CudaEngine:
         return out
 
     # ---- Minkowski p=2 on integer tokens: tcgen05 int8 contraction ---------------------------
-    GEMM_MAX_WIDTH = 256
+    # rows of up to 256 tokens keep their A tiles resident; wider rows stream K-chunks (pg_gemm.cu)
+    GEMM_MAX_WIDTH = 8192
 
     def gemm_pack(self, tokens, max_token=255, K=None):
         """(N, L) integer-valued tokens -> GemmTable; OverflowError if a value is not an integer
@@ -438,7 +439,7 @@ class CudaEngine:
         N, L_ = int(t.shape[0]), int(t.shape[1])
         K = int(self.lib.pg_gemm_width(L_)) if K is None else int(K)
         if K > self.GEMM_MAX_WIDTH:
-            raise L.Unsupported("rows wider than 256 tokens take the element-wise kernel")
+            raise L.Unsupported(f"rows wider than {self.GEMM_MAX_WIDTH} tokens take the element-wise kernel")
         rows_pad = int(self.lib.pg_gemm_rows(N))
         data = self.empty((rows_pad * K,), torch.uint8)
         norms = self.empty((rows_pad,), torch.int32)

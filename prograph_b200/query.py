@@ -104,7 +104,7 @@ def nearest(lib, queries, distance=hamming, group=None):
         except (OverflowError, L.Unsupported):
             part = None
     elif kind == "minkowski" and float(p) == 2.0 and lib.L <= eng.GEMM_MAX_WIDTH:
-        vk, max_token = gemm_value_kind(staged_dtype(_probe(lib.data), _probe(Qr), p))
+        vk, max_token = gemm_value_kind(staged_dtype(_probe(lib.data), _probe(Qr), p), lib.L)
         if vk is not None:
             try:
                 g = lib.gemm(max_token)
@@ -188,7 +188,7 @@ def _tiles(lib, Q, distance, kind, p, similarity, whole=False):
             yield b0, eng.hamming_values_tile(lib.device(dt), eng.to_device(Qb, dt), 0, Qb.shape[0], similarity=similarity)
         elif kind == "minkowski":
             dt = staged_dtype(_probe(lib.data), _probe(Qb), p)
-            vk, max_token = gemm_value_kind(dt)
+            vk, max_token = gemm_value_kind(dt, lib.L)
             if float(p) == 2.0 and vk is not None and lib.L <= eng.GEMM_MAX_WIDTH:
                 try:
                     g = lib.gemm(max_token)
