@@ -86,6 +86,10 @@ int pg_pack_chars(const uint8_t* chars, int64_t N, int L, int64_t ld, const uint
  * Fused Hamming sweeps: "own" rows live in registers, the "stream" table is swept
  * through shared memory; the (own x stream) distance matrix never reaches HBM.
  * Replaces hamming.py:34 + the consumer that follows it in prograph.py.
+ * Covered packed shapes (planes x words per plane, as pg_packed_words gives them): planes 5 or 8
+ * with words 1, 2, 4 and every multiple of 8 up to 1024 (rows of up to 32768 residues); other
+ * shapes return PG_ERR_UNSUPPORTED before any device work.  The symmetric sweeps below cover
+ * words <= 8, and 16 at 5 planes.
  * ------------------------------------------------------------------------- */
 
 /* size in bytes of the workspace the fused sweeps need (split partials) */
@@ -110,8 +114,8 @@ size_t pg_eps_workspace_bytes_capture(int64_t own_rows, int64_t stream_rows, int
  *   out_idx[r*k + j]  int64,  out_w[r*k + j] per `weight`.
  * If stream_rows < drop+k the tail is filled with idx = -1 and weight 0 (int64 0, or 0.0f for
  * similarities; the same for every kNN output of this library).  The lists of 256 own rows live in
- * shared memory: k + drop <= 78, fewer on rows of more than 1024 residues (their ring takes more
- * room), else PG_ERR_UNSUPPORTED.  */
+ * shared memory: k + drop <= 78 at every covered width except 5 planes with 1025..1792 residues
+ * (words 40..56, whose ring holds whole rows: fewer there), else PG_ERR_UNSUPPORTED.  */
 int pg_hamming_knn(const uint32_t* own, int64_t own_rows, int64_t row0, int64_t rows,
                    const uint32_t* stream_tab, int64_t stream_rows,
                    int planes, int words, int k, int drop, int weight,
@@ -207,7 +211,9 @@ size_t pg_eps_count_workspace_bytes(int64_t own_rows, int64_t stream_rows, int w
 /* epsilon graph, pass 1 (prograph.py:731-736): per own row, the number of stream rows
  * whose distance d has bit d set in `lut` (a host array of (L+32)/32 words: the
  * truth table of  comp(d, eps) & (d > 0)  -- or any other predicate of d -- evaluated
- * by the caller for d = 0..L).  counts[r] int64, r relative to row0.  */
+ * by the caller for d = 0..L).  lut_words <= 64 (distances up to 2047), and up to words + 1 for the
+ * rows of more than 1792 residues at 5 planes and more than 256 at 8 (copied to the device for
+ * the sweep).  counts[r] int64, r relative to row0.  */
 int pg_hamming_eps_count(const uint32_t* own, int64_t own_rows, int64_t row0, int64_t rows,
                          const uint32_t* stream_tab, int64_t stream_rows,
                          int planes, int words, const uint32_t* lut_host, int lut_words,

@@ -141,20 +141,28 @@ __global__ void select_rows_kernel(const uint32_t* __restrict__ mut, long long N
   }
 }
 
+// SHARED: per-block bins in shared memory, flushed with one global atomic per non-empty bin; rows too
+// long for the bins to fit in shared memory count straight into `hist`.
+template <bool SHARED>
 __global__ void distance_hist_kernel(const uint32_t* __restrict__ mut, long long N, int words, long long* __restrict__ hist,
                                      int bins) {
   extern __shared__ unsigned sh[];
-  for (int i = threadIdx.x; i < bins; i += blockDim.x) sh[i] = 0;
-  __syncthreads();
+  if (SHARED) {
+    for (int i = threadIdx.x; i < bins; i += blockDim.x) sh[i] = 0;
+    __syncthreads();
+  }
   for (long long n = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; n < N;
        n += static_cast<long long>(gridDim.x) * blockDim.x) {
     int d = 0;
     for (int w = 0; w < words; ++w) d += __popc(mut[static_cast<size_t>(n) * words + w]);
-    atomicAdd(&sh[d], 1u);
+    if (SHARED) atomicAdd(&sh[d], 1u);
+    else atomicAdd(reinterpret_cast<unsigned long long*>(hist + d), 1ull);
   }
-  __syncthreads();
-  for (int i = threadIdx.x; i < bins; i += blockDim.x)
-    if (sh[i]) atomicAdd(reinterpret_cast<unsigned long long*>(hist + i), static_cast<unsigned long long>(sh[i]));
+  if (SHARED) {
+    __syncthreads();
+    for (int i = threadIdx.x; i < bins; i += blockDim.x)
+      if (sh[i]) atomicAdd(reinterpret_cast<unsigned long long*>(hist + i), static_cast<unsigned long long>(sh[i]));
+  }
 }
 
 // Informative columns.  A thread walks the table with a stride that is a multiple of the row length,
@@ -317,6 +325,11 @@ int pg_varying_columns(const uint32_t* table, int64_t N, int planes, int words, 
   const long long stride = max(1ll, threads / row_elems) * row_elems;      // a multiple of the row length
   const unsigned grid = static_cast<unsigned>(ceil_div(stride, 256));
   const size_t smem = sizeof(uint32_t) * row_words;
+  if (smem > 48 * 1024) {       // one word per (plane, word) position: more than the default dynamic shared memory
+    PG_CUDA(cudaFuncSetAttribute(vec ? reinterpret_cast<const void*>(varying_columns_kernel<uint4>)
+                                     : reinterpret_cast<const void*>(varying_columns_kernel<uint32_t>),
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+  }
   if (vec)
     varying_columns_kernel<uint4><<<grid, 256, smem, s>>>(reinterpret_cast<const uint4*>(table), total, row_elems, stride,
                                                          varying);
@@ -335,6 +348,11 @@ int pg_compact_columns(const uint32_t* table, int64_t N, int planes, int words, 
   const size_t smem = sizeof(int) * out_words * 32;
   const unsigned grid = grid_for(rows_padded * out_words, 256);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (smem > 48 * 1024 && (planes == 5 || planes == 8)) {    // more than 384 output words: up to 128 KB
+    PG_CUDA(cudaFuncSetAttribute(planes == 5 ? reinterpret_cast<const void*>(compact_columns_kernel<5>)
+                                             : reinterpret_cast<const void*>(compact_columns_kernel<8>),
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+  }
   if (planes == 5)
     compact_columns_kernel<5><<<grid, 256, smem, s>>>(table, N, rows_padded, words, cols, out, out_words);
   else if (planes == 8)
@@ -407,8 +425,18 @@ int pg_flag_indices(const uint8_t* flag, int64_t N, int64_t* out_idx, int64_t* c
 int pg_distance_hist(const uint32_t* mut, int64_t N, int words, int64_t* hist, void* stream) {
   PG_CHECK_ARG(mut && hist && N > 0 && words > 0, "bad arguments");
   const int bins = words * 32 + 1;
-  distance_hist_kernel<<<grid_for(N, 256), 256, bins * sizeof(unsigned), static_cast<cudaStream_t>(stream)>>>(
-      mut, N, words, reinterpret_cast<long long*>(hist), bins);
+  const size_t smem = static_cast<size_t>(bins) * sizeof(unsigned);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (smem > 227 * 1024) {      // rows of more than 58 111 residues
+    distance_hist_kernel<false><<<grid_for(N, 256), 256, 0, s>>>(mut, N, words, reinterpret_cast<long long*>(hist), bins);
+    PG_LAUNCH_CHECK();
+    return PG_OK;
+  }
+  // bins of rows longer than 12 288 residues exceed the default 48 KB of dynamic shared memory
+  if (smem > 48 * 1024)
+    PG_CUDA(cudaFuncSetAttribute(distance_hist_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 static_cast<int>(smem)));
+  distance_hist_kernel<true><<<grid_for(N, 256), 256, smem, s>>>(mut, N, words, reinterpret_cast<long long*>(hist), bins);
   PG_LAUNCH_CHECK();
   return PG_OK;
 }

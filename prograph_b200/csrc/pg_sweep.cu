@@ -93,11 +93,18 @@ static Geometry make_geometry(long long rows, long long stream_rows, int words, 
 }
 
 int sweep_long_p5(const SweepParams& prm, const SweepLaunch& l, int words);   // pg_sweep_long.cu
+int sweep_wide_p5(const SweepParams& prm, const SweepLaunch& l, int words);   // pg_sweep_wide.cu
+int sweep_wide_p8(const SweepParams& prm, const SweepLaunch& l, int words);
 
 static bool long_rows(int planes, int words) { return planes == 5 && words > 16 && words <= 56 && words % 8 == 0; }
+// the chunked long-row sweep: P = 5 beyond 1792 residues, P = 8 beyond 256, both up to 32768
+static bool wide_rows(int planes, int words) {
+  return words % 8 == 0 && words <= kWideMaxWords && ((planes == 5 && words > 56) || (planes == 8 && words > 8));
+}
 
 static int dispatch(int planes, int words, const SweepParams& prm, const SweepLaunch& l) {
   if (long_rows(planes, words)) return sweep_long_p5(prm, l, words);
+  if (wide_rows(planes, words)) return planes == 5 ? sweep_wide_p5(prm, l, words) : sweep_wide_p8(prm, l, words);
 #define PG_CASE(P, W) \
   if (planes == P && words == W) return sweep_p##P##_w##W(prm, l);
   PG_CASE(5, 1) PG_CASE(5, 2) PG_CASE(5, 4) PG_CASE(5, 8) PG_CASE(5, 16)
@@ -117,9 +124,9 @@ static int check_common(const void* own, long long own_rows, long long row0, lon
   PG_CHECK_ARG((reinterpret_cast<uintptr_t>(str) & 15) == 0, "stream table must be 16-byte aligned");
   PG_CHECK_ARG((reinterpret_cast<uintptr_t>(own) & 15) == 0, "own table must be 16-byte aligned");
   if (!(((planes == 5 || planes == 8) && (words == 1 || words == 2 || words == 4 || words == 8)) ||
-        (planes == 5 && words == 16) || long_rows(planes, words))) {
-    set_error("fused sweep supports planes in {5,8} x words in {1,2,4,8} and planes=5 with words 16,24,..,56; got "
-              "planes=%d words=%d", planes, words);
+        (planes == 5 && words == 16) || long_rows(planes, words) || wide_rows(planes, words))) {
+    set_error("fused sweep supports planes in {5,8} x words in {1,2,4,8}, planes=5 with words 16,24,..,1024 and "
+              "planes=8 with words 16,24,..,1024; got planes=%d words=%d", planes, words);
     return PG_ERR_UNSUPPORTED;
   }
   return PG_OK;
@@ -768,7 +775,9 @@ static int eps_pass(int mode, const uint32_t* own, int64_t own_rows, int64_t row
                     void* workspace, size_t workspace_bytes, void* stream, int capture = 0) {
   int rc = check_common(own, own_rows, row0, rows, stream_tab, stream_rows, planes, words);
   if (rc != PG_OK) return rc;
-  PG_CHECK_ARG(lut_host && lut_words >= 1 && lut_words <= kMaxLutWords, "lut_words must be in [1,%d]", kMaxLutWords);
+  // the chunked sweep reads its truth table from shared memory: any table over d = 0..32*words
+  const int max_lut = wide_rows(planes, words) ? std::max(kMaxLutWords, words + 1) : kMaxLutWords;
+  PG_CHECK_ARG(lut_host && lut_words >= 1 && lut_words <= max_lut, "lut_words must be in [1,%d]", max_lut);
   PG_CHECK_ARG(lut_words * 32 > words * 32, "lut must cover distances 0..%d", words * 32);
   PG_CHECK_ARG(workspace, "null workspace");
   PG_CHECK_ARG(capture >= 0, "capture must be >= 0");
@@ -809,18 +818,31 @@ static int eps_pass(int mode, const uint32_t* own, int64_t own_rows, int64_t row
     prm.rows = n_over;
     prm.n_rowblocks = static_cast<int>(ceil_div(n_over, kConsumers));
   }
-  for (int i = 0; i < lut_words; ++i) prm.lut[i] = lut_host[i];
+  for (int i = 0; i < lut_words && i < kMaxLutWords; ++i) prm.lut[i] = lut_host[i];
   const bool ranged = lut_as_range(lut_host, lut_words, &prm.lo, &prm.span);
   SweepLaunch l{mode, ranged ? 0 : 1, weight, 0, 0, static_cast<cudaStream_t>(stream)};
+  l.lut_words = lut_words;
   if (mode == MODE_FILL) {
     prm.indptr = reinterpret_cast<const long long*>(indptr);
     prm.out_idx = reinterpret_cast<long long*>(out_idx);
     prm.out_w = out_w;
   }
+  void* lut_dev = nullptr;     // a table longer than the parameter block holds: device copy, freed in stream order
+  if (!ranged && lut_words > kMaxLutWords) {
+    PG_CUDA(temp_alloc(&lut_dev, sizeof(uint32_t) * lut_words, cs));
+    const cudaError_t e = cudaMemcpyAsync(lut_dev, lut_host, sizeof(uint32_t) * lut_words, cudaMemcpyHostToDevice, cs);
+    if (e != cudaSuccess) {
+      cudaFreeAsync(lut_dev, cs);
+      set_error("truth table upload failed: %s", cudaGetErrorString(e));
+      return PG_ERR_CUDA;
+    }
+    l.lut_ext = static_cast<const uint32_t*>(lut_dev);
+  }
   {
     SweepTimer t(l.stream);
     rc = dispatch(planes, words, prm, l);
   }
+  if (lut_dev != nullptr) cudaFreeAsync(lut_dev, cs);
   if (rc != PG_OK) return rc;
   if (mode == MODE_COUNT) {
     const int threads = 256;

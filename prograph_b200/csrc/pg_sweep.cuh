@@ -29,7 +29,9 @@ constexpr int kConsumerWarps = 8;
 constexpr int kConsumers = kConsumerWarps * 32;  // threads per CTA; each owns TM rows
 constexpr int kSweepThreads = kConsumers;
 constexpr int kStages = 4;
-constexpr int kMaxLutWords = 64;                 // distances up to 2047
+constexpr int kMaxLutWords = 64;                 // truth table in the parameter block: distances up to 2047
+                                                 // (the chunked long-row sweep takes longer ones: SweepLaunch::lut_ext)
+constexpr int kWideMaxWords = 1024;              // chunked long-row sweep: rows of up to 32768 residues
 constexpr int kEpsCapture = 128;                  // default hits per (split, row) kept by the count pass
 
 enum SweepMode { MODE_KNN = 0, MODE_COUNT = 1, MODE_FILL = 2, MODE_TILE = 3 };
@@ -474,6 +476,10 @@ struct SweepLaunch {
   size_t list_bytes;  // kNN lists (all own rows of a CTA)
   cudaStream_t stream;
   int rows_per_thread = 1;  // 2 selects the two-rows-per-thread kNN instantiation (experiments)
+  // chunked long-row sweep: the truth table (count / fill with lut = 1) has lut_words words, in
+  // SweepParams::lut when they fit, else in device memory at lut_ext
+  int lut_words = kMaxLutWords;
+  const uint32_t* lut_ext = nullptr;
 };
 
 template <int P, int W>

@@ -2,7 +2,7 @@
 import torch
 
 from .. import _lib as L
-from ..engine import get_engine
+from ..engine import get_engine, sweep_covers
 from .utils import clean_input, result_device, is_integer_dtype
 
 _QBLOCK = 512           # query rows per tile call: the packed stream-tile granularity
@@ -23,8 +23,8 @@ def hamming_matrix(eng, X, Y, similarity=False):
     try:
         xp = eng.pack(X)
         yp = eng.pack(Y, planes=xp.planes, words=xp.words)
-        if xp.words > 56 or (xp.words > 8 and xp.planes != 5):
-            raise L.Unsupported("rows longer than 1792 residues take the element-wise kernel")
+        if not sweep_covers(xp.planes, xp.words):
+            raise L.Unsupported("rows longer than 32768 residues take the element-wise kernel")
     except (OverflowError, L.Unsupported):
         # arbitrary numeric values: element-wise != on the device (IEEE: NaN differs from all)
         dt = value_dtype(torch.result_type(X, Y))

@@ -24,6 +24,16 @@ def _host_u32(a):
     return a, a.ctypes.data_as(C.c_void_p)
 
 
+SWEEP_MAX_WORDS = 1024     # 32768 residues per row: the longest rows the one-sided sweeps take
+
+
+def sweep_covers(planes, words):
+    """Whether the one-sided fused sweeps (pg_hamming_knn, _eps_*, _tile, _flags_tile) take a packed
+    table of `planes` bit planes and `words` 32-residue words per plane: every width pg_packed_words
+    gives up to 32768 residues, at 5 planes (alphabets of up to 31 tokens) and at 8 (up to 255)."""
+    return planes in (5, 8) and 1 <= words <= SWEEP_MAX_WORDS and (words in (1, 2, 4) or words % 8 == 0)
+
+
 class PackedTable:
     """Bit-plane token table on the device: int32 tensor [rows_padded, planes, words]."""
     __slots__ = ("data", "rows", "L", "planes", "words", "informative")

@@ -34,7 +34,7 @@ from . import _lib as L
 from . import shard as _shard
 from .distance.hamming import hamming, value_dtype
 from .distance.minkowski import minkowski, staged_dtype
-from .engine import get_engine
+from .engine import get_engine, sweep_covers
 from .trace import phase
 
 _CMP_CODES = {operator.lt: L.LT, operator.le: L.LE, operator.eq: L.EQ,
@@ -626,7 +626,7 @@ def build_neighbours(rep, eps=None, k=None, similarity=False, distance=hamming, 
     if packed is not None:
         with phase("columns"):
             packed = informative_table(eng, packed)     # may bring a wide table back into range
-    if packed is not None and (packed.words > 56 or (packed.words > 8 and packed.planes != 5)):
+    if packed is not None and not sweep_covers(packed.planes, packed.words):
         packed = None          # wider than the fused sweeps: element-wise tiles below
 
     if packed is not None:

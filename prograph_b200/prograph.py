@@ -30,7 +30,7 @@ from scipy import sparse
 from . import graph as _graph
 from .distance import hamming, minkowski  # noqa: F401  (re-exported for drop-in imports)
 from .distance.hamming import hamming_matrix
-from .engine import get_engine
+from .engine import get_engine, sweep_covers
 from .protein import Protein
 
 _MISSING = "This sequence is not in the dataset."
@@ -381,7 +381,8 @@ class Prograph:
             eng = get_engine()
             table = self._device_tokens()
             width = max(queries.shape[1], self.tokenized.shape[1])
-            if eng.packed_words(width) == table.words and queries.max(initial=0) < (1 << table.planes):
+            if eng.packed_words(width) == table.words and queries.max(initial=0) < (1 << table.planes) and \
+                    sweep_covers(table.planes, table.words):
                 q = eng.pack(queries, planes=table.planes, words=table.words)
                 idx, d = eng.hamming_knn(q, 0, q.rows, table, 1, drop=0)
                 idx, d = idx.cpu().numpy()[:, 0], d.cpu().numpy()[:, 0]
@@ -403,7 +404,8 @@ class Prograph:
         a frontier whose neighbourhood flags come out of ONE fused sweep (pg_hamming_flags_tile); the
         greedy order inside the frontier is then resolved on its batch x batch corner -- a frontier row
         that an earlier seed of the same batch covers is no seed -- and the member lists of the seeds are
-        compacted in one pass."""
+        compacted in one pass.  Sequences of more than 32768 residues are not covered by the fused sweep
+        and raise Unsupported."""
         eng = get_engine()
         table = self._device_tokens()
         n = len(self)

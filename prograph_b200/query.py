@@ -25,7 +25,7 @@ from . import _lib as L
 from . import shard as _shard
 from .distance.hamming import hamming
 from .distance.minkowski import gemm_value_kind, staged_dtype
-from .engine import get_engine
+from .engine import get_engine, sweep_covers
 from .graph import TILE_BUDGET_BYTES, _metric_kind, as_matrix, distance_lut
 from .trace import phase
 
@@ -47,8 +47,8 @@ class Library:
         """Bit planes of the dataset (raises OverflowError / Unsupported when it is not tokens)."""
         if self._packed is None:
             tab = self.eng.pack(self.data)
-            if tab.words > 56 or (tab.words > 8 and tab.planes != 5):
-                raise L.Unsupported("rows longer than 1792 residues take the element-wise kernels")
+            if not sweep_covers(tab.planes, tab.words):
+                raise L.Unsupported("rows longer than 32768 residues take the element-wise kernels")
             self._packed = tab
         return self._packed
 
