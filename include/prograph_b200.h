@@ -251,6 +251,28 @@ int pg_hamming_tile(const uint32_t* data, int64_t data_rows,
 int pg_exclusive_scan_i64(const int64_t* in, int64_t n, int64_t* out, void* stream);
 
 /* ---------------------------------------------------------------------------
+ * Growing a built graph by new rows (extend_neighbours): the old rows' stored neighbours joined
+ * with what a one-sided sweep found for them among the new rows, whose indices start at col_base.
+ * ------------------------------------------------------------------------- */
+/* kNN: for each of `rows` rows, merge the sorted list prev_idx/prev_w[r*ka ..) with the sorted
+ * candidates cand_idx/cand_w[r*kb ..) (cand indices + col_base) and write the first k entries to
+ * out_idx/out_w[r*k ..).  weight PG_W_I64: (distance asc, index asc); PG_W_SIM_F32: (similarity
+ * desc, index asc).  idx = -1 ends an input list; missing outputs get idx = -1 and weight 0 (0.0f).
+ * Any ka, kb >= 0 and k >= 1.  */
+int pg_knn_extend_merge(const int64_t* prev_idx, const void* prev_w, int ka,
+                        const int64_t* cand_idx, const void* cand_w, int kb,
+                        int64_t rows, int64_t col_base, int k, int weight,
+                        int64_t* out_idx, void* out_w, void* stream);
+/* epsilon: out row r = old row r followed by added row r with col_base added to its indices.
+ * The entries of row r of a part are idx[indptr[r] - indptr[0] ..) (row slices of a larger CSR are
+ * taken as they are); out_indptr[0] = 0, (rows+1) entries.  Weights int64 (PG_W_I64) or float32
+ * (PG_W_SIM_F32); out_idx / out_w hold the sum of both parts' entries.  */
+int pg_csr_append(const int64_t* old_indptr, const int64_t* old_idx, const void* old_w,
+                  const int64_t* add_indptr, const int64_t* add_idx, const void* add_w,
+                  int64_t rows, int64_t col_base, int weight,
+                  int64_t* out_indptr, int64_t* out_idx, void* out_w, void* stream);
+
+/* ---------------------------------------------------------------------------
  * Element-wise metric tiles (float / generic values).
  * ------------------------------------------------------------------------- */
 /* minkowski.py:36-40.  X [N][D], Y [M][D] of `dtype` in {PG_F16, PG_F32, PG_F64, PG_I64};

@@ -13,10 +13,10 @@ _lib.load()   # fail loudly at import time when libprograph_b200.so has not been
 from .distance import hamming, minkowski, clean_input  # noqa: E402
 from .protein import Protein  # noqa: E402
 from .prograph import Prograph  # noqa: E402
-from .graph import build_neighbours, NeighbourTable, KnnTable  # noqa: E402
+from .graph import build_neighbours, extend_neighbours, NeighbourTable, KnnTable  # noqa: E402
 from .io import save  # noqa: E402
 from . import query  # noqa: E402,F401  (distance-to-dataset queries fused with their consumers)
 
-__all__ = ["Prograph", "Protein", "hamming", "minkowski", "clean_input", "build_neighbours",
+__all__ = ["Prograph", "Protein", "hamming", "minkowski", "clean_input", "build_neighbours", "extend_neighbours",
            "NeighbourTable", "KnnTable", "save", "query"]
 __version__ = "0.1.0"

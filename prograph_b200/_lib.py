@@ -64,6 +64,8 @@ SIGNATURES = {
     "pg_hamming_flags_tile": (_i, [_vp, _i64, _vp, _i64, _i64, _i64, _i, _i, _i, _i, _vp, _i64, _vp]),
     "pg_flags_or_rows": (_i, [_vp, _i64, _i64, _i64, _vp, _vp, _vp]),
     "pg_exclusive_scan_i64": (_i, [_vp, _i64, _vp, _vp]),
+    "pg_knn_extend_merge": (_i, [_vp, _vp, _i, _vp, _vp, _i, _i64, _i64, _i, _i, _vp, _vp, _vp]),
+    "pg_csr_append": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i, _vp, _vp, _vp, _vp]),
     "pg_minkowski_tile": (_i, [_vp, _i64, _vp, _i64, _i64, _i64, _i, _i, _dbl, _i, _vp, _i64, _vp]),
     "pg_hamming_values_tile": (_i, [_vp, _i64, _vp, _i64, _i64, _i64, _i, _i, _i, _vp, _i64, _vp]),
     "pg_gemm_width": (_i, [_i]),

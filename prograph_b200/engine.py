@@ -260,6 +260,40 @@ class CudaEngine:
                                             self._stream()))
         return out
 
+    def knn_extend_merge(self, prev_idx, prev_w, cand_idx, cand_w, col_base, k, similarity=False):
+        """(rows, k) kNN lists of rows whose sorted lists `prev_*` (rows, kA) meet sorted candidates
+        `cand_*` (rows, kB) from a table whose row 0 is row `col_base` of the graph
+        (pg_knn_extend_merge): the first k of the merge in (distance, index) order."""
+        rows, ka = prev_idx.shape
+        kb = cand_idx.shape[1]
+        wdt = torch.float32 if similarity else torch.int64
+        prev_idx, prev_w = prev_idx.contiguous(), prev_w.to(wdt).contiguous()
+        cand_idx, cand_w = cand_idx.contiguous(), cand_w.to(wdt).contiguous()
+        idx = self.empty((rows, k), torch.int64)
+        w = self.empty((rows, k), wdt)
+        L.check(self.lib.pg_knn_extend_merge(_ptr(prev_idx), _ptr(prev_w), ka, _ptr(cand_idx), _ptr(cand_w), kb, rows,
+                                             int(col_base), int(k), L.W_SIM_F32 if similarity else L.W_I64, _ptr(idx),
+                                             _ptr(w), self._stream()))
+        return idx, w
+
+    def csr_append(self, old, add, col_base, similarity=False):
+        """CSR whose row r is row r of `old` followed by row r of `add` with `col_base` added to its
+        indices (pg_csr_append).  Both are (indptr, idx, w) of the same rows; an indptr may start
+        above 0 (a row slice of a larger CSR whose idx / w are cut to those rows)."""
+        wdt = torch.float32 if similarity else torch.int64
+        (oip, oi, ow), (aip, ai, aw) = ([t.contiguous() for t in part[:2]] + [part[2].to(wdt).contiguous()]
+                                        for part in (old, add))
+        rows = oip.numel() - 1
+        nnz = oi.numel() + ai.numel()
+        self.check_edge_budget(nnz)
+        indptr = self.empty((rows + 1,), torch.int64)
+        idx = self.empty((nnz,), torch.int64)
+        w = self.empty((nnz,), wdt)
+        L.check(self.lib.pg_csr_append(_ptr(oip), _ptr(oi), _ptr(ow), _ptr(aip), _ptr(ai), _ptr(aw),
+                                       rows, int(col_base), L.W_SIM_F32 if similarity else L.W_I64, _ptr(indptr),
+                                       _ptr(idx), _ptr(w), self._stream()))
+        return indptr, idx, w
+
     def hamming_eps(self, own, row0, rows, stream, lut, similarity=False, capture=None):
         """prograph.py:731-753 for own rows [row0,row0+rows): CSR (indptr, idx, w) of the
         stream rows whose distance d has bit d set in `lut` (uint32 words, host).  `capture`:

@@ -362,11 +362,11 @@ def _hamming_knn_sym(eng, packed, kk, similarity, rank, world, group, output):
     return out + (0,)
 
 
-def hamming_knn_tiles(eng, own, stream, k, similarity, row0, rows):
+def hamming_knn_tiles(eng, own, stream, k, similarity, row0, rows, drop=1):
     """Same result through materialised int64 tiles + the tile top-k: used when k is too large
     for the in-shared-memory lists of the fused sweep.  Ascending distance with index ties is
     the same order as descending similarity, so the sort always runs on the distances."""
-    kk = min(k, stream.rows - 1)
+    kk = min(k, stream.rows - drop)
     step = max(512, (TILE_BUDGET_BYTES // (8 * stream.rows)) // 512 * 512)
     idxs, ws = [], []
     a0 = row0 // 512 * 512
@@ -374,7 +374,7 @@ def hamming_knn_tiles(eng, own, stream, k, similarity, row0, rows):
         qn = min(step, own.rows - q0)
         tile = eng.hamming_tile(stream, own, q0, qn, weight=L.W_I64)
         lo, hi = max(row0, q0) - q0, min(row0 + rows, q0 + qn) - q0
-        i, d = eng.tile_topk(tile[lo:hi], kk, drop=1, descending=False)
+        i, d = eng.tile_topk(tile[lo:hi], kk, drop=drop, descending=False)
         idxs.append(i)
         ws.append(1 / (1 + d) if similarity else d)        # hamming.py:38, on the device
     return torch.cat(idxs), torch.cat(ws)
@@ -685,3 +685,157 @@ def build_neighbours(rep, eps=None, k=None, similarity=False, distance=hamming, 
         return NeighbourTable(_to_host(indptr), _to_host(idx), _to_host(w), row0=row0 if sharded_out else 0)
     idx, w = part if sharded_out else _shard.gather_rows(part, n, rank, world, group, eng)
     return KnnTable(_to_host(idx), _to_host(w), row0=row0 if sharded_out else 0)
+
+
+# ---------------------------------------------------------------------------------
+# growing a built graph by new rows
+# ---------------------------------------------------------------------------------
+def stack_rows(A, B):
+    """`A` over `B`, the narrower side right-padded with token 0 (the clean_input rule,
+    distance/utils.py): a position padded in both rows of a pair adds nothing to their distance."""
+    width = max(A.shape[1], B.shape[1])
+    if isinstance(A, torch.Tensor) or isinstance(B, torch.Tensor):
+        dev = A.device if isinstance(A, torch.Tensor) else B.device
+        A, B = (torch.as_tensor(t).to(dev) for t in (A, B))
+        return torch.cat([torch.nn.functional.pad(t, (0, width - t.shape[1])) for t in (A, B)])
+    return np.concatenate([np.pad(t, ((0, 0), (0, width - t.shape[1]))) for t in (A, B)])
+
+
+def _check_previous(table, n_old, eps, k):
+    if eps and not isinstance(table, NeighbourTable):
+        raise ValueError("an epsilon graph is extended from the NeighbourTable its build returned")
+    if not eps and not isinstance(table, KnnTable):
+        raise ValueError("a kNN graph is extended from the KnnTable its build returned")
+    if table.row0 != 0 or table.n_rows != n_old:
+        raise ValueError(f"table must hold the whole graph of rep ({n_old} rows from row 0), not rows "
+                         f"[{table.row0}, {table.row0 + table.n_rows}): gather a sharded build first")
+    if not eps and table.idx.shape[1] != min(k, n_old - 1):
+        raise ValueError(f"table has {table.idx.shape[1]} neighbours per row, a build of {n_old} rows with "
+                         f"k={k} has {min(k, n_old - 1)}")
+
+
+def _upload(eng, a):
+    return torch.from_numpy(np.ascontiguousarray(a)).to(eng.device)
+
+
+def _extend_knn_rows(eng, table, packed, fresh, kk, similarity, a, b, col_base):
+    """kNN lists of old rows [a, b) in the grown graph: the stored lists merged with the rows'
+    candidates among the new rows.  Position 0 of an old row is itself or a lower-indexed duplicate,
+    never a new row (indices >= col_base), so the stored positions 1..k and the new candidates hold
+    the grown row's positions 1..kk."""
+    kc = min(kk, fresh.rows)
+    try:
+        ci, cw = eng.hamming_knn(packed, a, b - a, fresh, kc, drop=0, similarity=similarity)
+    except L.Unsupported:
+        ci, cw = hamming_knn_tiles(eng, packed, fresh, kc, similarity, a, b - a, drop=0)
+    with phase("upload"):
+        pi, pw = _upload(eng, table.idx[a:b]), _upload(eng, table.w[a:b])
+    with phase("merge"):
+        return eng.knn_extend_merge(pi, pw, ci, cw, col_base, kk, similarity)
+
+
+def _extend_eps_rows(eng, table, packed, fresh, lut, similarity, a, b, col_base):
+    """Epsilon rows [a, b) in the grown graph: the stored rows followed by their edges to the new
+    rows, which all have larger indices."""
+    add = hamming_eps_device(eng, packed, fresh, lut, similarity, a, b - a)
+    with phase("upload"):
+        ip = table.indptr[a:b + 1]
+        lo, hi = int(ip[0]), int(ip[-1])
+        old = (_upload(eng, ip), _upload(eng, table.idx[lo:hi]), _upload(eng, table.w[lo:hi]))
+    with phase("merge"):
+        return eng.csr_append(old, add, col_base, similarity)
+
+
+def _cat_csr(parts):
+    if len(parts) == 1:
+        return parts[0]
+    (ip0, i0, w0), (ip1, i1, w1) = parts
+    return torch.cat([ip0, ip1[1:] - ip1[0] + ip0[-1]]), torch.cat([i0, i1]), torch.cat([w0, w1])
+
+
+def extend_neighbours(table, rep, new, eps=None, k=None, similarity=False, distance=hamming, comp=operator.le,
+                      engine=None, group=None, output="replicated"):
+    """The graph of `rep` stacked over `new` from `table`, the graph ``build_neighbours(rep, eps|k,
+    similarity, distance, comp)`` returned (whole: row0 0, one row per row of rep), without sweeping
+    the old x old pairs again.  The result is bit for bit ``build_neighbours(concat, ...)`` with
+    the same arguments and `output`, where `concat` is rep over new with the narrower side
+    right-padded with token 0 (as clean_input pads): CSR arrays or kNN lists, dtypes and tie order.
+
+    Hamming on integer tokens within the fused sweeps: each old row is swept against the new rows
+    only and joined with its stored row (pg_knn_extend_merge / pg_csr_append); the new rows are
+    swept against the whole grown table, 2NM + M^2 pair evaluations instead of (N+M)^2.  The ranks
+    of a process group split the grown rows as a build does.  Every other metric or value type is
+    a rebuild of the concatenation."""
+    validate(eps, k)
+    if output not in ("replicated", "sharded"):
+        raise ValueError("output must be 'replicated' or 'sharded'")
+    A, B = as_matrix(rep), as_matrix(new)
+    n_old, m = A.shape[0], B.shape[0]
+    if m == 0:
+        raise ValueError("no new rows to add")
+    if n_old == 0:
+        raise ValueError("empty representation")
+    _check_previous(table, n_old, eps, k)
+    X = stack_rows(A, B)
+    n = n_old + m
+    eng = engine if engine is not None else get_engine()
+    rank, world = _shard.rank_world(group)
+    packed = None
+    if _metric_kind(distance)[0] == "hamming":
+        try:
+            with phase("pack"):
+                packed = pack_table(eng, X, rank, world, group)
+        except OverflowError:
+            packed = None
+    if packed is not None:
+        with phase("columns"):
+            # over the grown table: a position constant over the old rows may vary over the new ones
+            packed = informative_table(eng, packed)
+    if packed is None or not sweep_covers(packed.planes, packed.words):
+        return build_neighbours(X, eps=eps, k=k, similarity=similarity, distance=distance, comp=comp, engine=eng,
+                                group=group, output=output)
+    wdt = np.dtype(np.float32 if similarity else np.int64)
+    if np.asarray(table.w).dtype != wdt:
+        raise ValueError(f"table weights are {np.asarray(table.w).dtype}; a build with similarity={similarity} "
+                         f"gives {wdt}")
+    with phase("columns"):
+        fresh = eng.gather_packed(packed, np.arange(n_old, n))      # the new rows, same columns
+    row0, rows = _shard.row_range(n, rank, world)
+    old_rows = (row0, min(row0 + rows, n_old))                      # this rank's rows of each part
+    new_rows = (max(row0, n_old), row0 + rows)
+    sharded = world > 1 and n >= world
+    if eps:
+        lut = distance_lut(packed.words * 32, comp, 1 / (1 + eps) if similarity else eps, similarity)
+        code, exc, parts = _shard.OK, None, []
+        try:
+            with phase("sweep"):
+                if old_rows[1] > old_rows[0]:
+                    parts.append(_extend_eps_rows(eng, table, packed, fresh, lut, similarity, *old_rows, n_old))
+                if new_rows[1] > new_rows[0]:
+                    a, b = new_rows
+                    parts.append(hamming_eps_device(eng, packed, packed, lut, similarity, a, b - a))
+        except MemoryError as e:
+            code, exc = _shard.NO_MEMORY, e
+        _raise_code(_shard.agree(code, world, group, eng.device) if sharded else code, exc)
+        part = _cat_csr(parts)
+        if output != "sharded":
+            with phase("gather"):
+                part = _shard.gather_csr(part, n, rank, world, group, eng)
+            row0 = 0
+        with phase("d2h"):
+            return NeighbourTable(*(_to_host(t) for t in part), row0=row0)
+    kk = min(k, n - 1)
+    parts = []
+    with phase("sweep"):
+        if old_rows[1] > old_rows[0]:
+            parts.append(_extend_knn_rows(eng, table, packed, fresh, kk, similarity, *old_rows, n_old))
+        if new_rows[1] > new_rows[0]:
+            a, b = new_rows
+            parts.append(hamming_knn_device(eng, packed, packed, k, similarity, a, b - a))
+    part = tuple(torch.cat(t) for t in zip(*parts))
+    if output != "sharded":
+        with phase("gather"):
+            part = _shard.gather_rows(part, n, rank, world, group, eng)
+        row0 = 0
+    with phase("d2h"):
+        return KnnTable(_to_host(part[0]), _to_host(part[1]), row0=row0)
