@@ -96,22 +96,40 @@ int sweep_long_p5(const SweepParams& prm, const SweepLaunch& l, int words);   //
 int sweep_wide_p5(const SweepParams& prm, const SweepLaunch& l, int words);   // pg_sweep_wide.cu
 int sweep_wide_p8(const SweepParams& prm, const SweepLaunch& l, int words);
 
-static bool long_rows(int planes, int words) { return planes == 5 && words > 16 && words <= 56 && words % 8 == 0; }
-// the chunked long-row sweep: P = 5 beyond 1792 residues, P = 8 beyond 256, both up to 32768
-static bool wide_rows(int planes, int words) {
-  return words % 8 == 0 && words <= kWideMaxWords && ((planes == 5 && words > 56) || (planes == 8 && words > 8));
+// Which sweep covers rows of `planes` bit planes x `words` words: the own row in registers
+// (pg_sweep.cuh, also the only shapes of the symmetric sweep), whole stream rows of up to 1792
+// residues in the ring (pg_sweep_long.cu), or the chunked ring up to 32768 residues (pg_sweep_wide.cu).
+enum SweepPath { PATH_NONE, PATH_REGISTER, PATH_LONG, PATH_CHUNKED };
+
+static SweepPath sweep_path(int planes, int words) {
+  if (planes != 5 && planes != 8) return PATH_NONE;
+  if (words == 1 || words == 2 || words == 4 || words == 8 || (planes == 5 && words == 16)) return PATH_REGISTER;
+  if (words % 8 != 0 || words > kWideMaxWords) return PATH_NONE;
+  if (planes == 5 && words > 16 && words <= 56) return PATH_LONG;
+  if ((planes == 5 && words > 56) || (planes == 8 && words > 8)) return PATH_CHUNKED;
+  return PATH_NONE;
+}
+
+static int unsupported_shape(int planes, int words) {
+  set_error("fused sweep supports planes in {5,8} x words in {1,2,4,8}, planes=5 with words 16,24,..,1024 and "
+            "planes=8 with words 16,24,..,1024; got planes=%d words=%d", planes, words);
+  return PG_ERR_UNSUPPORTED;
 }
 
 static int dispatch(int planes, int words, const SweepParams& prm, const SweepLaunch& l) {
-  if (long_rows(planes, words)) return sweep_long_p5(prm, l, words);
-  if (wide_rows(planes, words)) return planes == 5 ? sweep_wide_p5(prm, l, words) : sweep_wide_p8(prm, l, words);
+  switch (sweep_path(planes, words)) {
+    case PATH_LONG: return sweep_long_p5(prm, l, words);
+    case PATH_CHUNKED: return planes == 5 ? sweep_wide_p5(prm, l, words) : sweep_wide_p8(prm, l, words);
+    case PATH_REGISTER:
 #define PG_CASE(P, W) \
   if (planes == P && words == W) return sweep_p##P##_w##W(prm, l);
-  PG_CASE(5, 1) PG_CASE(5, 2) PG_CASE(5, 4) PG_CASE(5, 8) PG_CASE(5, 16)
-  PG_CASE(8, 1) PG_CASE(8, 2) PG_CASE(8, 4) PG_CASE(8, 8)
+      PG_CASE(5, 1) PG_CASE(5, 2) PG_CASE(5, 4) PG_CASE(5, 8) PG_CASE(5, 16)
+      PG_CASE(8, 1) PG_CASE(8, 2) PG_CASE(8, 4) PG_CASE(8, 8)
 #undef PG_CASE
-  set_error("fused sweep supports planes in {5,8} and words in {1,2,4,8}; got planes=%d words=%d", planes, words);
-  return PG_ERR_UNSUPPORTED;
+      break;
+    case PATH_NONE: break;
+  }
+  return unsupported_shape(planes, words);
 }
 
 static int check_common(const void* own, long long own_rows, long long row0, long long rows, const void* str,
@@ -123,12 +141,7 @@ static int check_common(const void* own, long long own_rows, long long row0, lon
   PG_CHECK_ARG(stream_rows < (1ll << 32), "stream table too large for 32-bit indices");
   PG_CHECK_ARG((reinterpret_cast<uintptr_t>(str) & 15) == 0, "stream table must be 16-byte aligned");
   PG_CHECK_ARG((reinterpret_cast<uintptr_t>(own) & 15) == 0, "own table must be 16-byte aligned");
-  if (!(((planes == 5 || planes == 8) && (words == 1 || words == 2 || words == 4 || words == 8)) ||
-        (planes == 5 && words == 16) || long_rows(planes, words) || wide_rows(planes, words))) {
-    set_error("fused sweep supports planes in {5,8} x words in {1,2,4,8}, planes=5 with words 16,24,..,1024 and "
-              "planes=8 with words 16,24,..,1024; got planes=%d words=%d", planes, words);
-    return PG_ERR_UNSUPPORTED;
-  }
+  if (sweep_path(planes, words) == PATH_NONE) return unsupported_shape(planes, words);
   return PG_OK;
 }
 
@@ -202,39 +215,53 @@ __device__ __forceinline__ void flush_rows(const unsigned long long* sm, long lo
 static int rows_per_merge_block(int kk) { return kk <= 32 ? 128 : 32; }
 static size_t merge_smem_bytes(int kk) { return static_cast<size_t>(rows_per_merge_block(kk)) * (kk + 1) * 8; }
 
-// ---- kNN: merge the per-split lists, drop leading entries, widen ---------------------
-__global__ void knn_finalize_kernel(const unsigned long long* __restrict__ part, int n_splits, int k1, long long rows,
-                                    int k, int drop, int weight, long long* __restrict__ out_idx, void* out_w) {
+// ---- kNN: merge sorted key lists per row, drop leading entries, keep the keys or widen ----------
+// Entry i of list s of row r is lists[s * list_stride + r * row_stride + i * entry_stride]: the split
+// lists of the one-sided sweep are [s][i][row], the lists of the ranks [s][row][i].  Keys are unique
+// (index in the low word), so "smallest key above the last one" walks the merged order; each list is
+// ascending, so its scan stops at the first usable entry.  A single list is copied through.
+__global__ void knn_merge_scan_kernel(const unsigned long long* __restrict__ lists, int n_lists, long long list_stride,
+                                      long long row_stride, long long entry_stride, long long rows, int k1, int k,
+                                      int drop, int weight, bool keys_out, unsigned long long* __restrict__ out_keys,
+                                      long long* __restrict__ out_idx, void* out_w) {
   extern __shared__ unsigned long long merge_sm[];
   const long long row_base = blockIdx.x * static_cast<long long>(blockDim.x);
   const long long r = row_base + threadIdx.x;
   unsigned long long* mine = merge_sm + threadIdx.x * (k + 1);
   if (r < rows) {
+    const unsigned long long* row = lists + r * row_stride;
     unsigned long long last = 0;
-    bool have_last = false;
     for (int j = 0; j < drop + k; ++j) {
       unsigned long long best = ~0ull;
-      if (n_splits == 1) {
-        best = j < k1 ? part[static_cast<size_t>(j) * rows + r] : ~0ull;
-      } else {
-        // keys are unique (index in the low word), so "smallest key above the last one" walks
-        // the merged order; each split list is ascending, stop at the first usable entry
-        for (int s = 0; s < n_splits; ++s) {
-          const unsigned long long* lst = part + static_cast<size_t>(s) * k1 * rows + r;
+      if (n_lists == 1) {
+        best = j < k1 ? row[j * entry_stride] : ~0ull;
+      } else if (j == 0 || last != ~0ull) {     // nothing follows the end of every list
+        for (int s = 0; s < n_lists; ++s) {
+          const unsigned long long* lst = row + s * list_stride;
           for (int i = 0; i < k1; ++i) {
-            const unsigned long long v = lst[static_cast<size_t>(i) * rows];
-            if (have_last && v <= last) continue;
+            const unsigned long long v = lst[i * entry_stride];
+            if (j > 0 && v <= last) continue;
             if (v < best) best = v;
             break;
           }
         }
       }
       last = best;
-      have_last = true;
       if (j >= drop) mine[j - drop] = best;
     }
   }
-  flush_rows(merge_sm, row_base, rows, k, weight, false, nullptr, out_idx, out_w);
+  flush_rows(merge_sm, row_base, rows, k, weight, keys_out, out_keys, out_idx, out_w);
+}
+
+static int knn_merge_scan(const unsigned long long* lists, int n_lists, long long list_stride, long long row_stride,
+                          long long entry_stride, long long rows, int k1, int k, int drop, int weight,
+                          unsigned long long* out_keys, long long* out_idx, void* out_w, cudaStream_t stream) {
+  const int threads = rows_per_merge_block(k);
+  knn_merge_scan_kernel<<<static_cast<unsigned>(ceil_div(rows, threads)), threads, merge_smem_bytes(k), stream>>>(
+      lists, n_lists, list_stride, row_stride, entry_stride, rows, k1, k, drop, weight, out_keys != nullptr, out_keys,
+      out_idx, out_w);
+  PG_LAUNCH_CHECK();
+  return PG_OK;
 }
 
 __global__ void sum_splits_kernel(const long long* __restrict__ split_counts, int n_splits, long long rows,
@@ -328,20 +355,20 @@ static size_t eps_plan_bytes(const EpsPlan& p, long long rows) {
 
 
 // ---- symmetric kNN sweep (pg_sweep_sym.cuh): host side ---------------------------------
+// the symmetric sweep keeps the own row in registers: the shapes of PATH_REGISTER
+static bool sym_shape_ok(int planes, int words) { return sweep_path(planes, words) == PATH_REGISTER; }
+
 static int dispatch_sym(int planes, int words, const SymParams& prm, const SymLaunch& l, int* resident) {
+  if (sym_shape_ok(planes, words)) {
 #define PG_CASE(P, W) \
   if (planes == P && words == W) return sweep_sym_p##P##_w##W(prm, l, resident);
-  PG_CASE(5, 1) PG_CASE(5, 2) PG_CASE(5, 4) PG_CASE(5, 8) PG_CASE(5, 16)
-  PG_CASE(8, 1) PG_CASE(8, 2) PG_CASE(8, 4) PG_CASE(8, 8)
+    PG_CASE(5, 1) PG_CASE(5, 2) PG_CASE(5, 4) PG_CASE(5, 8) PG_CASE(5, 16)
+    PG_CASE(8, 1) PG_CASE(8, 2) PG_CASE(8, 4) PG_CASE(8, 8)
 #undef PG_CASE
+  }
   set_error("symmetric sweep supports planes in {5,8} x words in {1,2,4,8} and planes=5, words=16; got planes=%d "
             "words=%d", planes, words);
   return PG_ERR_UNSUPPORTED;
-}
-
-static bool sym_shape_ok(int planes, int words) {
-  return ((planes == 5 || planes == 8) && (words == 1 || words == 2 || words == 4 || words == 8)) ||
-         (planes == 5 && words == 16);
 }
 
 // workspace: [filter words: tiles*tile_cols u64][locks: rows u32][stats: 8 u64, error word at +64 B][items]
@@ -533,37 +560,6 @@ __global__ void sym_init_kernel(unsigned long long* glist, long long n_keys, uns
   for (long long j = i; j < rows; j += stride) glock[j] = 0u;
 }
 
-// bootstrap: merged split lists [n_splits][k1][rows] -> row-major key lists [rows][k1]
-__global__ void knn_part_to_lists_kernel(const unsigned long long* __restrict__ part, int n_splits, int k1,
-                                         long long rows, unsigned long long* __restrict__ lists) {
-  extern __shared__ unsigned long long merge_sm[];
-  const long long row_base = blockIdx.x * static_cast<long long>(blockDim.x);
-  const long long r = row_base + threadIdx.x;
-  unsigned long long* mine = merge_sm + threadIdx.x * (k1 + 1);
-  if (r < rows) {
-    unsigned long long last = 0;
-    bool ended = false;
-    for (int j = 0; j < k1; ++j) {
-      unsigned long long best = ~0ull;
-      if (!ended) {
-        for (int s = 0; s < n_splits; ++s) {
-          const unsigned long long* lst = part + static_cast<size_t>(s) * k1 * rows + r;
-          for (int i = 0; i < k1; ++i) {
-            const unsigned long long v = lst[static_cast<size_t>(i) * rows];
-            if (j > 0 && v <= last) continue;
-            if (v < best) best = v;
-            break;
-          }
-        }
-      }
-      last = best;
-      ended |= best == ~0ull;
-      mine[j] = best;
-    }
-  }
-  flush_rows(merge_sm, row_base, rows, k1, PG_W_I64, true, lists, nullptr, nullptr);
-}
-
 // Final lists: merge n_lists sorted key lists per row (one per rank), drop, then either widen to the
 // reference's (index int64, weight) arrays or keep the merged keys (KEYS_OUT: the exchange step of the
 // multi-GPU build all-gathers 8-byte keys and widens locally).  Every list keeps a cursor and its
@@ -601,38 +597,6 @@ __global__ void knn_lists_finalize_kernel(const unsigned long long* __restrict__
           }
         }
       }
-      if (j >= drop) mine[j - drop] = best;
-    }
-  }
-  flush_rows(merge_sm, row_base, rows, k, weight, keys_out, out_keys, out_idx, out_w);
-}
-
-// more lists than cursors fit in registers: "smallest key above the last one", rescanning the lists
-__global__ void knn_lists_finalize_scan_kernel(const unsigned long long* __restrict__ lists, int n_lists,
-                                               long long list_stride, long long row0, long long rows, int k1, int k,
-                                               int drop, int weight, bool keys_out,
-                                               unsigned long long* __restrict__ out_keys, long long* __restrict__ out_idx,
-                                               void* out_w) {
-  extern __shared__ unsigned long long merge_sm[];
-  const long long row_base = blockIdx.x * static_cast<long long>(blockDim.x);
-  const long long r = row_base + threadIdx.x;
-  unsigned long long* mine = merge_sm + threadIdx.x * (k + 1);
-  if (r < rows) {
-    unsigned long long last = 0;
-    bool have_last = false;
-    for (int j = 0; j < drop + k; ++j) {
-      unsigned long long best = ~0ull;
-      for (int s = 0; s < n_lists; ++s) {
-        const unsigned long long* lst = lists + static_cast<size_t>(s) * list_stride + static_cast<size_t>(row0 + r) * k1;
-        for (int i = 0; i < k1; ++i) {
-          const unsigned long long v = lst[i];
-          if (have_last && v <= last) continue;
-          if (v < best) best = v;
-          break;
-        }
-      }
-      last = best;
-      have_last = true;
       if (j >= drop) mine[j - drop] = best;
     }
   }
@@ -700,14 +664,9 @@ extern "C" {
 size_t pg_sweep_workspace_bytes(int64_t own_rows, int64_t stream_rows, int words, int k1) {
   if (own_rows <= 0 || stream_rows <= 0 || words <= 0) return 0;
   // the largest split count any sweep of this shape may choose (kNN with k1 entries, the
-  // count / fill passes, the two-rows-per-thread kNN variants)
-  int n_splits = 1;
-  for (int rpc = kConsumers; rpc <= 2 * kConsumers; rpc += kConsumers) {
-    const int a = make_geometry(own_rows, stream_rows, words, rpc, 0).n_splits;
-    const int b = make_geometry(own_rows, stream_rows, words, rpc, k1 > 0 ? k1 : 1).n_splits;
-    n_splits = a > n_splits ? a : n_splits;
-    n_splits = b > n_splits ? b : n_splits;
-  }
+  // count / fill passes)
+  const int n_splits = std::max(make_geometry(own_rows, stream_rows, words, kConsumers, 0).n_splits,
+                                make_geometry(own_rows, stream_rows, words, kConsumers, k1 > 0 ? k1 : 1).n_splits);
   const size_t per_row = static_cast<size_t>(n_splits) * 8 * static_cast<size_t>(k1 > 1 ? k1 : 1);
   return per_row * static_cast<size_t>(own_rows) + 256;
 }
@@ -737,16 +696,10 @@ int pg_hamming_knn(const uint32_t* own, int64_t own_rows, int64_t row0, int64_t 
   PG_CHECK_ARG(out_idx && out_w && workspace, "null output/workspace pointer");
   PG_CHECK_ARG(weight == PG_W_I64 || weight == PG_W_SIM_F32 || weight == PG_W_I32, "bad weight kind %d", weight);
   const int k1 = drop + k;
-  // experiment knob: PG_KNN_VARIANT=1 runs two own rows per thread (planes 5, words 8 only)
-  int tm = 1;
-  int variant = 0;
-  if (const char* ev = std::getenv("PG_KNN_VARIANT")) variant = std::atoi(ev);
-  if (!(planes == 5 && words == 8)) variant = 0;
-  if (variant == 1 || variant == 4) tm = 2;
-  const Geometry g = make_geometry(rows, stream_rows, words, kConsumers * tm, k1);
+  const Geometry g = make_geometry(rows, stream_rows, words, kConsumers, k1);
   const size_t need = static_cast<size_t>(g.n_splits) * k1 * rows * 8;
   PG_CHECK_ARG(workspace_bytes >= need, "workspace too small: %zu < %zu", workspace_bytes, need);
-  const size_t list_bytes = static_cast<size_t>(k1) * kConsumers * tm * 8;
+  const size_t list_bytes = static_cast<size_t>(k1) * kConsumers * 8;
   if (k1 > 32 * kMaxListRounds || list_bytes + 70 * 1024 > 227 * 1024) {
     set_error("k=%d too large for the in-shared-memory lists of the fused sweep", k);
     return PG_ERR_UNSUPPORTED;
@@ -755,18 +708,14 @@ int pg_hamming_knn(const uint32_t* own, int64_t own_rows, int64_t row0, int64_t 
   fill_common(prm, g, own, row0, rows, stream_tab, stream_rows);
   prm.part = static_cast<unsigned long long*>(workspace);
   prm.k1 = k1;
-  SweepLaunch l{MODE_KNN, 0, weight, 0, list_bytes, static_cast<cudaStream_t>(stream)};
-  l.rows_per_thread = variant == 3 ? 3 : (variant == 4 ? 4 : tm);
+  SweepLaunch l{MODE_KNN, 0, weight, list_bytes, static_cast<cudaStream_t>(stream)};
   {
     SweepTimer t(l.stream);
     rc = dispatch(planes, words, prm, l);
   }
   if (rc != PG_OK) return rc;
-  const int threads = rows_per_merge_block(k);
-  knn_finalize_kernel<<<static_cast<unsigned>(ceil_div(rows, threads)), threads, merge_smem_bytes(k), l.stream>>>(
-      prm.part, g.n_splits, k1, rows, k, drop, weight, reinterpret_cast<long long*>(out_idx), out_w);
-  PG_LAUNCH_CHECK();
-  return PG_OK;
+  return knn_merge_scan(prm.part, g.n_splits, static_cast<long long>(k1) * rows, 1, rows, rows, k1, k, drop, weight,
+                        nullptr, reinterpret_cast<long long*>(out_idx), out_w, l.stream);
 }
 
 static int eps_pass(int mode, const uint32_t* own, int64_t own_rows, int64_t row0, int64_t rows,
@@ -776,7 +725,7 @@ static int eps_pass(int mode, const uint32_t* own, int64_t own_rows, int64_t row
   int rc = check_common(own, own_rows, row0, rows, stream_tab, stream_rows, planes, words);
   if (rc != PG_OK) return rc;
   // the chunked sweep reads its truth table from shared memory: any table over d = 0..32*words
-  const int max_lut = wide_rows(planes, words) ? std::max(kMaxLutWords, words + 1) : kMaxLutWords;
+  const int max_lut = sweep_path(planes, words) == PATH_CHUNKED ? std::max(kMaxLutWords, words + 1) : kMaxLutWords;
   PG_CHECK_ARG(lut_host && lut_words >= 1 && lut_words <= max_lut, "lut_words must be in [1,%d]", max_lut);
   PG_CHECK_ARG(lut_words * 32 > words * 32, "lut must cover distances 0..%d", words * 32);
   PG_CHECK_ARG(workspace, "null workspace");
@@ -820,7 +769,7 @@ static int eps_pass(int mode, const uint32_t* own, int64_t own_rows, int64_t row
   }
   for (int i = 0; i < lut_words && i < kMaxLutWords; ++i) prm.lut[i] = lut_host[i];
   const bool ranged = lut_as_range(lut_host, lut_words, &prm.lo, &prm.span);
-  SweepLaunch l{mode, ranged ? 0 : 1, weight, 0, 0, static_cast<cudaStream_t>(stream)};
+  SweepLaunch l{mode, ranged ? 0 : 1, weight, 0, static_cast<cudaStream_t>(stream)};
   l.lut_words = lut_words;
   if (mode == MODE_FILL) {
     prm.indptr = reinterpret_cast<const long long*>(indptr);
@@ -922,7 +871,7 @@ int pg_hamming_tile(const uint32_t* data, int64_t data_rows, const uint32_t* que
   fill_common(prm, g, data, 0, data_rows, queries + static_cast<size_t>(q0) * planes * words, qrows);
   prm.out = out;
   prm.ld = ld;
-  SweepLaunch l{MODE_TILE, 0, weight, 0, 0, static_cast<cudaStream_t>(stream)};
+  SweepLaunch l{MODE_TILE, 0, weight, 0, static_cast<cudaStream_t>(stream)};
   SweepTimer t(l.stream);
   return dispatch(planes, words, prm, l);
 }
@@ -945,7 +894,7 @@ int pg_hamming_flags_tile(const uint32_t* data, int64_t data_rows, const uint32_
   prm.lo = d_lo;
   prm.span = d_hi >= d_lo ? static_cast<unsigned>(d_hi - d_lo) : 0u;
   if (d_hi < d_lo) prm.lo = 0x7fffffff;               // empty range: nothing passes
-  SweepLaunch l{MODE_TILE, 0, PG_W_FLAG_U8, 0, 0, static_cast<cudaStream_t>(stream)};
+  SweepLaunch l{MODE_TILE, 0, PG_W_FLAG_U8, 0, static_cast<cudaStream_t>(stream)};
   SweepTimer t(l.stream);
   return dispatch(planes, words, prm, l);
 }
@@ -973,17 +922,15 @@ int pg_hamming_knn_boot(const uint32_t* table, int64_t table_rows, int64_t row0,
   fill_common(prm, g, table, row0, rows, table, boot_rows);
   prm.part = static_cast<unsigned long long*>(workspace);
   prm.k1 = k1;
-  SweepLaunch l{MODE_KNN, 0, PG_W_I64, 0, static_cast<size_t>(k1) * kConsumers * 8, static_cast<cudaStream_t>(stream)};
+  SweepLaunch l{MODE_KNN, 0, PG_W_I64, static_cast<size_t>(k1) * kConsumers * 8, static_cast<cudaStream_t>(stream)};
   {
     SweepTimer t(l.stream);
     rc = dispatch(planes, words, prm, l);
   }
   if (rc != PG_OK) return rc;
-  const int threads = rows_per_merge_block(k1);
-  knn_part_to_lists_kernel<<<static_cast<unsigned>(ceil_div(rows, threads)), threads, merge_smem_bytes(k1), l.stream>>>(
-      prm.part, g.n_splits, k1, rows, reinterpret_cast<unsigned long long*>(lists));
-  PG_LAUNCH_CHECK();
-  return PG_OK;
+  // merged split lists [n_splits][k1][rows] -> row-major key lists [rows][k1]
+  return knn_merge_scan(prm.part, g.n_splits, static_cast<long long>(k1) * rows, 1, rows, rows, k1, k1, 0, PG_W_I64,
+                        reinterpret_cast<unsigned long long*>(lists), nullptr, nullptr, l.stream);
 }
 
 int pg_knn_sym_band(int64_t rows, int words, int64_t boot_rows, int part, int parts, int64_t* row_begin,
@@ -1203,9 +1150,6 @@ static int knn_lists_launch(const uint64_t* lists, int n_lists, int64_t list_str
   PG_CHECK_ARG(lists && (out_keys || (out_idx && out_w)), "null pointer");
   PG_CHECK_ARG(n_lists >= 1 && rows > 0 && row0 >= 0 && k >= 1 && drop >= 0 && k1 >= 1, "bad list geometry");
   PG_CHECK_ARG(weight == PG_W_I64 || weight == PG_W_SIM_F32 || weight == PG_W_I32, "bad weight kind %d", weight);
-  const int threads = rows_per_merge_block(k);
-  const size_t msm = merge_smem_bytes(k);
-  const unsigned grid = static_cast<unsigned>(ceil_div(rows, threads));
   cudaStream_t cs = static_cast<cudaStream_t>(stream);
   const unsigned long long* src = reinterpret_cast<const unsigned long long*>(lists);
   unsigned long long* ok = reinterpret_cast<unsigned long long*>(out_keys);
@@ -1214,12 +1158,14 @@ static int knn_lists_launch(const uint64_t* lists, int n_lists, int64_t list_str
     knn_keys_widen_kernel<<<static_cast<unsigned>(blocks), 256, 0, cs>>>(src, row0, rows, k1, k, drop, weight,
                                                                         reinterpret_cast<long long*>(out_idx), out_w);
   } else if (n_lists <= kMaxMergeLists) {
-    knn_lists_finalize_kernel<<<grid, threads, msm, cs>>>(src, n_lists, list_stride, row0, rows, k1, k, drop, weight,
-                                                        out_keys != nullptr, ok, reinterpret_cast<long long*>(out_idx), out_w);
+    const int threads = rows_per_merge_block(k);
+    knn_lists_finalize_kernel<<<static_cast<unsigned>(ceil_div(rows, threads)), threads, merge_smem_bytes(k), cs>>>(
+        src, n_lists, list_stride, row0, rows, k1, k, drop, weight, out_keys != nullptr, ok,
+        reinterpret_cast<long long*>(out_idx), out_w);
   } else {
-    knn_lists_finalize_scan_kernel<<<grid, threads, msm, cs>>>(src, n_lists, list_stride, row0, rows, k1, k, drop, weight,
-                                                             out_keys != nullptr, ok, reinterpret_cast<long long*>(out_idx),
-                                                             out_w);
+    // more lists than cursors fit in registers: rescan them
+    return knn_merge_scan(src + row0 * k1, n_lists, list_stride, k1, 1, rows, k1, k, drop, weight, ok,
+                          reinterpret_cast<long long*>(out_idx), out_w, cs);
   }
   PG_LAUNCH_CHECK();
   return PG_OK;

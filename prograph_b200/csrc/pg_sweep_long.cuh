@@ -99,7 +99,6 @@ __global__ void __launch_bounds__(kSweepThreads, 2) sweep_long_kernel(const __gr
   unsigned long long* lists = reinterpret_cast<unsigned long long*>(lut_s + lut_room);   // [256][k1]
 
   const int tid = threadIdx.x;
-  const int warp = tid >> 5;
   const int lane = tid & 31;
 
   // the work-item cursor counts ring tiles of LBN rows here; CHUNKED: (tile, chunk) units, la_c the chunk
@@ -107,71 +106,48 @@ __global__ void __launch_bounds__(kSweepThreads, 2) sweep_long_kernel(const __gr
   la.start(blockIdx.x, prm);
   const int n_wide = CHUNKED ? (Wt + kWideChunk - 1) / kWideChunk : 1;
   int la_c = 0;
-  if (tid == 0) {
-    for (int s = 0; s < n_stages; ++s) {
-      mbar_init(&full[s], 1);
-      done[s] = 0;
-    }
-    fence_mbar_init();
-  }
-  if constexpr (CHUNKED) {
-    if (LUT) {
-      const uint32_t* src = wide.lut_ext != nullptr ? wide.lut_ext : prm.lut;
-      for (int i = tid; i < wide.lut_words; i += kSweepThreads) lut_s[i] = src[i];
-    }
-  } else {
-    if (LUT && tid < kMaxLutWords) lut_s[tid] = prm.lut[tid];
-  }
-  __syncthreads();
-#pragma unroll 1
-  for (int s = 0; s < n_stages; ++s) {
+  auto more = [&] { return la.valid(prm); };
+  auto issue = [&](int s) {
     if constexpr (CHUNKED) {
-      if (warp == 0 && la.valid(prm))
-        issue_wide_unit<P>(stage_mem + static_cast<size_t>(s) * WIDE_STAGE_WORDS, &full[s], prm.str, Wt, la.t, la_c, lane);
+      issue_wide_unit<P>(stage_mem + static_cast<size_t>(s) * WIDE_STAGE_WORDS, &full[s], prm.str, Wt, la.t, la_c, lane);
+    } else {
+      mbar_arrive_expect_tx(&full[s], STAGE_BYTES);
+      bulk_g2s(stage_mem + static_cast<size_t>(s) * LBN * COLW, prm.str + static_cast<size_t>(la.t) * LBN * COLW,
+               STAGE_BYTES, &full[s]);
+    }
+  };
+  auto step = [&] {
+    if constexpr (CHUNKED) {
       if (la.valid(prm) && ++la_c == n_wide) { la_c = 0; la.advance(prm, gridDim.x); }
     } else {
-      if (tid == 0 && la.valid(prm)) {
-        mbar_arrive_expect_tx(&full[s], STAGE_BYTES);
-        bulk_g2s(stage_mem + static_cast<size_t>(s) * LBN * COLW, prm.str + static_cast<size_t>(la.t) * LBN * COLW,
-                 STAGE_BYTES, &full[s]);
-      }
       if (la.valid(prm)) la.advance(prm, gridDim.x);
     }
-  }
+  };
+  auto load_lut = [&] {
+    if constexpr (CHUNKED) {
+      if (LUT) {
+        const uint32_t* src = wide.lut_ext != nullptr ? wide.lut_ext : prm.lut;
+        for (int i = tid; i < wide.lut_words; i += kSweepThreads) lut_s[i] = src[i];
+      }
+    } else {
+      if (LUT && tid < kMaxLutWords) lut_s[tid] = prm.lut[tid];
+    }
+  };
+  ring_start<CHUNKED>(full, done, n_stages, tid, load_lut, more, issue, step);
 
   const int n_items = prm.n_rowblocks * prm.n_splits;
   const int n_chunks = Wt / LCH;
   const unsigned one = prm.one;
-  const int lo = prm.lo;
-  const unsigned span = prm.span;
   int stage = 0;
   uint32_t phase = 0;
+  // the pad rows at the table end carry 0x3fffffff, beyond every truth table: LUT tests are bounded
+  SweepEpilogue<MODE, LUT, WEIGHT, true> ep{prm, lists, lut_s, (CHUNKED ? wide.lut_words : kMaxLutWords) * 32, tid};
 
   for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
     const int split = item / prm.n_rowblocks;
-    const int rb = item - split * prm.n_rowblocks;
-    long long r = static_cast<long long>(rb) * kConsumers + tid;
-    const bool valid = r < prm.rows;
-    if (prm.row_map != nullptr && valid) r = prm.row_map[r];
-    const uint32_t* ownp = prm.own + static_cast<size_t>(prm.own_row0 + (valid ? r : 0)) * COLW;
-    unsigned tau = valid ? 0xffffffffu : 0u;
-    long long cnt = 0;
-    unsigned long long* cap = nullptr;
-    unsigned long long* my_list = lists + static_cast<size_t>(tid) * prm.k1;
-    if constexpr (MODE == MODE_KNN) {
-      for (int j = 0; j < prm.k1; ++j) my_list[j] = ~0ull;
-      __syncwarp();
-    }
-    if constexpr (MODE == MODE_COUNT) {
-      if (valid && prm.capture != nullptr)
-        cap = prm.capture + (static_cast<size_t>(split) * prm.rows_total + r) * prm.capture_cap;
-    }
-    if constexpr (MODE == MODE_FILL) {
-      if (valid) {
-        cnt = prm.indptr[r];
-        for (int s = 0; s < split; ++s) cnt += prm.split_counts[static_cast<size_t>(s) * prm.rows_total + r];
-      }
-    }
+    ep.begin(item - split * prm.n_rowblocks, split);
+    const uint32_t* ownp = prm.own + ep.own_row() * COLW;
+    if constexpr (MODE == MODE_KNN) __syncwarp();
 
     const int t0 = split * prm.tiles_per_split;
     const int t1 = min(t0 + prm.tiles_per_split, prm.n_tiles);
@@ -206,20 +182,7 @@ __global__ void __launch_bounds__(kSweepThreads, 2) sweep_long_kernel(const __gr
             for (int j = 0; j < LBN; ++j) acc[j] += ham_chunk<P, SUB>(q, unit + j * P * cw + h, cw, one);
           }
           // done with this unit: the last warp to get here refills the stage with the lookahead unit
-          __syncwarp();
-          unsigned last = 0;
-          if (lane == 0) last = atom_add_acq_rel_cta(&done[stage], 1u) == kConsumerWarps - 1;
-          last = __shfl_sync(0xffffffffu, last, 0);
-          if (last) {
-            if (lane == 0) done[stage] = 0;
-            if (la.valid(prm)) {
-              fence_proxy_async();
-              issue_wide_unit<P>(stage_mem + static_cast<size_t>(stage) * WIDE_STAGE_WORDS, &full[stage], prm.str, Wt,
-                                 la.t, la_c, lane);
-            }
-          }
-          if (la.valid(prm) && ++la_c == n_wide) { la_c = 0; la.advance(prm, gridDim.x); }
-          if (++stage == n_stages) { stage = 0; phase ^= 1u; }
+          ring_release<true>(done, stage, phase, n_stages, lane, more, issue, step);
         }
       } else {
 #pragma unroll 1
@@ -248,79 +211,18 @@ __global__ void __launch_bounds__(kSweepThreads, 2) sweep_long_kernel(const __gr
       if constexpr (MODE == MODE_KNN) {
 #pragma unroll
         for (int g = 0; g < LBN / 4; ++g) {
-          const unsigned best = min(min(static_cast<unsigned>(acc[4 * g]), static_cast<unsigned>(acc[4 * g + 1])),
-                                    min(static_cast<unsigned>(acc[4 * g + 2]), static_cast<unsigned>(acc[4 * g + 3])));
-          if (__any_sync(0xffffffffu, best < tau)) {
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-              const int dv = acc[4 * g + e];
-              unsigned cand = __ballot_sync(0xffffffffu, static_cast<unsigned>(dv) < tau);
-              while (cand) {
-                const int src = __ffs(cand) - 1;
-                cand &= cand - 1;
-                const unsigned dd = __shfl_sync(0xffffffffu, static_cast<unsigned>(dv), src);
-                const unsigned long long key =
-                    (static_cast<unsigned long long>(dd) << 32) | static_cast<unsigned>(col0 + 4 * g + e);
-                const unsigned t_new =
-                    knn_insert_coop(lists + static_cast<size_t>((warp << 5) + src) * prm.k1, prm.k1, key, lane);
-                if (lane == src) tau = t_new;
-              }
-            }
-          }
+          const int d[4] = {acc[4 * g], acc[4 * g + 1], acc[4 * g + 2], acc[4 * g + 3]};
+          ep.offer4(d, col0 + 4 * g);
         }
       } else {
 #pragma unroll
-        for (int j = 0; j < LBN; ++j) {
-          const int d = acc[j];
-          if constexpr (MODE == MODE_TILE) {
-            if (valid && j < ncols) write_tile<WEIGHT>(prm.out, (col0 + j) * prm.ld + r, d, prm.lo, prm.span);
-          } else {
-            bool hit;
-            if constexpr (LUT && CHUNKED) hit = d < wide.lut_words * 32 && ((lut_s[d >> 5] >> (d & 31)) & 1u);
-            else if constexpr (LUT) hit = d < kMaxLutWords * 32 && ((lut_s[d >> 5] >> (d & 31)) & 1u);
-            else hit = static_cast<unsigned>(d - lo) <= span;
-            if (hit && valid) {
-              if constexpr (MODE == MODE_COUNT) {
-                if (cap != nullptr && cnt < prm.capture_cap)
-                  cap[cnt] = (static_cast<unsigned long long>(static_cast<unsigned>(d)) << 32) |
-                             static_cast<unsigned>(col0 + j);
-              } else {
-                prm.out_idx[cnt] = col0 + j;
-                write_weight(prm.out_w, cnt, d, WEIGHT);
-              }
-              ++cnt;
-            }
-          }
-        }
+        for (int j = 0; j < LBN; ++j)
+          if (MODE != MODE_TILE || j < ncols) ep.offer(acc[j], col0 + j);
       }
 
-      if constexpr (!CHUNKED) {
-        __syncwarp();
-        if (lane == 0) {
-          if (atom_add_acq_rel_cta(&done[stage], 1u) == kConsumerWarps - 1) {
-            done[stage] = 0;
-            if (la.valid(prm)) {
-              fence_proxy_async();
-              mbar_arrive_expect_tx(&full[stage], STAGE_BYTES);
-              bulk_g2s(stage_mem + static_cast<size_t>(stage) * LBN * COLW,
-                       prm.str + static_cast<size_t>(la.t) * LBN * COLW, STAGE_BYTES, &full[stage]);
-            }
-          }
-        }
-        if (la.valid(prm)) la.advance(prm, gridDim.x);
-        if (++stage == LSTAGES) { stage = 0; phase ^= 1u; }
-      }
+      if constexpr (!CHUNKED) ring_release(done, stage, phase, LSTAGES, lane, more, issue, step);
     }
-
-    if constexpr (MODE == MODE_KNN) {
-      if (valid) {
-        unsigned long long* dst = prm.part + static_cast<size_t>(split) * prm.k1 * prm.rows_total + r;
-        for (int j = 0; j < prm.k1; ++j) dst[static_cast<size_t>(j) * prm.rows_total] = my_list[j];
-      }
-      __syncwarp();
-    } else if constexpr (MODE == MODE_COUNT) {
-      if (valid) prm.split_counts[static_cast<size_t>(split) * prm.rows_total + r] = cnt;
-    }
+    ep.end();
   }
 }
 
@@ -337,9 +239,9 @@ static int launch_long_one(const SweepParams& prm, const SweepLaunch& l, int Wt)
   auto kern = sweep_long_kernel<P, MODE, LUT, WEIGHT, CHUNKED>;
   WideArgs wide{l.lut_ext, l.lut_words, 0};
   size_t smem = 0;
-  int occ = 0;
   if constexpr (CHUNKED) {
     // 3 stages unless 2 give more CTAs per SM (long kNN lists) or 3 do not fit at all
+    int occ = 0;
     for (int st = LSTAGES; st >= 2; --st) {
       const size_t b = wide_smem_bytes<P, MODE, LUT>(l, st);
       if (b > 227 * 1024) continue;
@@ -349,46 +251,22 @@ static int launch_long_one(const SweepParams& prm, const SweepLaunch& l, int Wt)
       if (o > occ) { occ = o; smem = b; wide.stages = st; }
     }
     if (wide.stages == 0) { set_error("chunked long-row sweep does not fit in shared memory"); return PG_ERR_UNSUPPORTED; }
-    PG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   } else {
     smem = static_cast<size_t>(LSTAGES) * LBN * P * Wt * 4 + 2 * kStages * sizeof(uint64_t) + kMaxLutWords * 4 +
            l.list_bytes;
     if (smem > 227 * 1024) { set_error("long-row sweep does not fit in shared memory (%zu bytes)", smem); return PG_ERR_UNSUPPORTED; }
-    PG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    PG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kSweepThreads, smem));
   }
-  if (occ < 1) { set_error("long-row sweep does not fit on an SM"); return PG_ERR_UNSUPPORTED; }
-  const long long n_items = static_cast<long long>(prm.n_rowblocks) * prm.n_splits;
-  long long grid = static_cast<long long>(num_sms()) * occ;
-  if (grid > n_items) grid = n_items;
-  if (grid < 1) grid = 1;
-  kern<<<static_cast<unsigned>(grid), kSweepThreads, smem, l.stream>>>(prm, Wt, wide);
-  PG_LAUNCH_CHECK();
-  return PG_OK;
+  return launch_persistent(kern, smem, static_cast<long long>(prm.n_rowblocks) * prm.n_splits, l.stream, nullptr, prm, Wt,
+                           wide);
 }
 
 // Every mode and weight of the long-row sweep at P planes; CHUNKED selects the chunked ring.
 template <int P, bool CHUNKED>
 static int launch_long(const SweepParams& prm, const SweepLaunch& l, int words) {
-  switch (l.mode) {
-    case MODE_KNN: return launch_long_one<P, MODE_KNN, false, 0, CHUNKED>(prm, l, words);
-    case MODE_COUNT:
-      return l.lut ? launch_long_one<P, MODE_COUNT, true, 0, CHUNKED>(prm, l, words)
-                   : launch_long_one<P, MODE_COUNT, false, 0, CHUNKED>(prm, l, words);
-    case MODE_FILL:
-      if (l.weight == PG_W_SIM_F32)
-        return l.lut ? launch_long_one<P, MODE_FILL, true, PG_W_SIM_F32, CHUNKED>(prm, l, words)
-                     : launch_long_one<P, MODE_FILL, false, PG_W_SIM_F32, CHUNKED>(prm, l, words);
-      return l.lut ? launch_long_one<P, MODE_FILL, true, PG_W_I64, CHUNKED>(prm, l, words)
-                   : launch_long_one<P, MODE_FILL, false, PG_W_I64, CHUNKED>(prm, l, words);
-    case MODE_TILE:
-      if (l.weight == PG_W_I64) return launch_long_one<P, MODE_TILE, false, PG_W_I64, CHUNKED>(prm, l, words);
-      if (l.weight == PG_W_SIM_F32) return launch_long_one<P, MODE_TILE, false, PG_W_SIM_F32, CHUNKED>(prm, l, words);
-      if (l.weight == PG_W_FLAG_U8) return launch_long_one<P, MODE_TILE, false, PG_W_FLAG_U8, CHUNKED>(prm, l, words);
-      return launch_long_one<P, MODE_TILE, false, PG_W_I32, CHUNKED>(prm, l, words);
-  }
-  set_error("bad sweep mode %d", l.mode);
-  return PG_ERR_INVALID;
+  return with_sweep_variant(l, [&](auto v) {
+    using V = decltype(v);
+    return launch_long_one<P, V::mode, V::lut, V::weight, CHUNKED>(prm, l, words);
+  });
 }
 
 }  // namespace pg

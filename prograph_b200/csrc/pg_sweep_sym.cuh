@@ -246,30 +246,18 @@ __global__ void __launch_bounds__(kSweepThreads, 2) sweep_sym_kernel(const __gri
   const int k1 = prm.k1;
   unsigned long long* warp_lists = lists + static_cast<size_t>(warp << 5) * k1;
 
-  auto fill_stage = [&](int s, int t) {   // one elected thread: tile t (and its filter words) into ring stage s
-    mbar_arrive_expect_tx(&full[s], STAGE_BYTES + TAU_BYTES);
-    bulk_g2s(stage_mem + s * (BN * COLW), prm.tab + static_cast<size_t>(t) * BN * COLW, STAGE_BYTES, &full[s]);
-    if constexpr (MODE == SYM_KNN) bulk_g2s(taus + s * BN, prm.glast + static_cast<size_t>(t) * BN, TAU_BYTES, &full[s]);
-  };
-
   const int item_first = __ldg(prm.cta_first + blockIdx.x), item_end = __ldg(prm.cta_first + blockIdx.x + 1);
   SymCursor la;
   la.end = item_end;
   la.start(item_first, prm);
-  if (tid == 0) {
-#pragma unroll
-    for (int s = 0; s < kStages; ++s) {
-      mbar_init(&full[s], 1);
-      done[s] = 0;
-    }
-    fence_mbar_init();
-  }
-  __syncthreads();
-#pragma unroll 1
-  for (int s = 0; s < kStages; ++s) {
-    if (tid == 0 && la.valid()) fill_stage(s, la.t);
-    if (la.valid()) la.advance(prm);
-  }
+  auto more = [&] { return la.valid(); };
+  auto issue = [&](int s) {   // tile la.t (and its filter words) into ring stage s
+    mbar_arrive_expect_tx(&full[s], STAGE_BYTES + TAU_BYTES);
+    bulk_g2s(stage_mem + s * (BN * COLW), prm.tab + static_cast<size_t>(la.t) * BN * COLW, STAGE_BYTES, &full[s]);
+    if constexpr (MODE == SYM_KNN) bulk_g2s(taus + s * BN, prm.glast + static_cast<size_t>(la.t) * BN, TAU_BYTES, &full[s]);
+  };
+  auto step = [&] { if (la.valid()) la.advance(prm); };
+  ring_start(full, done, kStages, tid, [] {}, more, issue, step);
 
   int stage = 0;
   uint32_t phase = 0;
@@ -291,13 +279,6 @@ __global__ void __launch_bounds__(kSweepThreads, 2) sweep_sym_kernel(const __gri
 #pragma unroll
       for (int j = 0; j < COLW; ++j) q[j] = valid ? __ldg(src + j) : 0u;
     }
-    const uint32_t(&qq)[1][COLW] = reinterpret_cast<const uint32_t(&)[1][COLW]>(q);
-    // distance of the own row to the stream row at `col` (shared memory, broadcast loads)
-    auto dist = [&](const uint32_t* col) -> int {
-      int d[1];
-      ham_rows<P, W, 1>(qq, col, d, one);
-      return d[0];
-    };
     // kNN: the row's global list already bounds what can still matter: ties at its last distance
     // stay admissible (the index decides), hence the +1
     int tau_seed = 0, tau = 0;
@@ -388,28 +369,16 @@ __global__ void __launch_bounds__(kSweepThreads, 2) sweep_sym_kernel(const __gri
 
 #pragma unroll 1
       for (; c + 4 <= ncols; c += 4) {
-        int d0[1], d1[1], d2[1], d3[1];
-        ham_rows4<P, W, 1>(qq, tile + c * COLW, d0, d1, d2, d3, one);
-        vote(c, d0[0], d1[0], d2[0], d3[0]);
+        int d[4];
+        ham_rows4<P, W>(q, tile + c * COLW, d, one);
+        vote(c, d[0], d[1], d[2], d[3]);
       }
 #pragma unroll 1
       for (; c < ncols; ++c) {   // ragged end of the table (last tile only)
-        const int d = dist(tile + c * COLW);
-        rare(d, c, c >= c_mid);
+        rare(ham_rows<P, W>(q, tile + c * COLW, one), c, c >= c_mid);
       }
 
-      __syncwarp();
-      if (lane == 0) {
-        if (atom_add_acq_rel_cta(&done[stage], 1u) == kConsumerWarps - 1) {
-          done[stage] = 0;
-          if (la.valid()) {
-            fence_proxy_async();
-            fill_stage(stage, la.t);
-          }
-        }
-      }
-      if (la.valid()) la.advance(prm);
-      if (++stage == kStages) { stage = 0; phase ^= 1u; }
+      ring_release(done, stage, phase, kStages, lane, more, issue, step);
     }
 
     if constexpr (MODE == SYM_KNN) {
@@ -439,23 +408,14 @@ struct SymLaunch {
   int mode = SYM_KNN;
 };
 
-
-// grid == 0: only report the resident grid (CTAs) through *resident
+// grid == 0: only report the resident grid (CTAs) through *resident; otherwise grid is the CTA count
+// of a plan made for at most that many CTAs, so launch_persistent launches all of them
 template <int P, int W, int MODE>
 int launch_sweep_sym_mode(const SymParams& prm, const SymLaunch& l, int* resident) {
-  auto kern = sweep_sym_kernel<P, W, MODE>;
   const size_t smem = static_cast<size_t>(kStages) * (TileCols<W>::value * P * W * 4 +
                                                       (MODE == SYM_KNN ? TileCols<W>::value * 8 : 0)) +
                       2 * kStages * sizeof(uint64_t) + l.list_bytes;
-  PG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-  int occ = 0;
-  PG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kSweepThreads, smem));
-  if (occ < 1) { set_error("symmetric sweep does not fit on an SM (smem %zu bytes)", smem); return PG_ERR_UNSUPPORTED; }
-  if (resident) *resident = num_sms() * occ;
-  if (l.grid <= 0) return PG_OK;
-  kern<<<static_cast<unsigned>(l.grid), kSweepThreads, smem, l.stream>>>(prm);
-  PG_LAUNCH_CHECK();
-  return PG_OK;
+  return launch_persistent(sweep_sym_kernel<P, W, MODE>, smem, l.grid, l.stream, resident, prm);
 }
 
 template <int P, int W>

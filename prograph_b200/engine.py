@@ -183,7 +183,7 @@ class CudaEngine:
 
     SYM_MAX_LIST = 32      # list length (k + drop) the symmetric sweep keeps per row
 
-    def _sym_check(self, table, k1):
+    def _sym_check(self, table, k1=1):
         if k1 > self.SYM_MAX_LIST or table.words > 16 or (table.words > 8 and table.planes != 5):
             raise L.Unsupported("shape not covered by the symmetric sweep")
 
@@ -346,7 +346,8 @@ class CudaEngine:
         unordered pairs; returns (keys, edges): the reserved slots of the edge-key buffer (both
         directions of every passing pair, sentinels -1 in unused slots) and the number of edges
         among them.  Raises Unsupported when `lut` is not one contiguous range of distances."""
-        if table.words > 16 or (table.words > 8 and table.planes != 5) or table.rows >= (1 << 27):
+        self._sym_check(table)
+        if table.rows >= (1 << 27):
             raise L.Unsupported("shape not covered by the symmetric sweep")
         lut, lut_p = _host_u32(lut)
         nbytes = int(self.lib.pg_knn_sym_workspace_bytes(table.rows, table.words))

@@ -1,14 +1,13 @@
 #!/usr/bin/env python3
-"""Time the fused Hamming kNN sweep (and its experimental variants) on one GPU.
+"""Time the fused Hamming kNN sweep on one GPU.
 
-    python tools/profile_knn.py --n 262144 --variants 0,1,2,3,4
-Used under ncu for the profiles committed in profiles/ (one variant, small --n).
+    python tools/profile_knn.py --n 262144
+Used under ncu for the profiles committed in profiles/ (small --n).
 """
 import argparse
 import os
 import sys
 
-import numpy as np
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -19,7 +18,6 @@ def main():
     ap.add_argument("--n", type=int, default=262144)
     ap.add_argument("--length", type=int, default=256)
     ap.add_argument("--k", type=int, default=16)
-    ap.add_argument("--variants", default="0")
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--dist", default="uniform")
     args = ap.parse_args()
@@ -28,26 +26,17 @@ def main():
     eng = get_engine()
     X = make_tokens(args.n, args.length, args.dist)
     tab = eng.pack(X)
-    ref = None
-    for v in [int(x) for x in args.variants.split(",")]:
-        os.environ["PG_KNN_VARIANT"] = str(v)
-        idx, w = eng.hamming_knn(tab, 0, args.n, tab, args.k, drop=1)      # warm-up + result
+    eng.hamming_knn(tab, 0, args.n, tab, args.k, drop=1)      # warm-up
+    torch.cuda.synchronize()
+    best = 1e30
+    for _ in range(args.reps):
+        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a.record()
+        eng.hamming_knn(tab, 0, args.n, tab, args.k, drop=1)
+        b.record()
         torch.cuda.synchronize()
-        best = 1e30
-        for _ in range(args.reps):
-            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            a.record()
-            eng.hamming_knn(tab, 0, args.n, tab, args.k, drop=1)
-            b.record()
-            torch.cuda.synchronize()
-            best = min(best, a.elapsed_time(b))
-        same = ""
-        if ref is None:
-            ref = (idx.clone(), w.clone())
-        else:
-            same = f" same_as_v0={bool(torch.equal(idx, ref[0]) and torch.equal(w, ref[1]))}"
-        print(f"variant {v}: {best:.2f} ms  {args.n * args.n / best / 1e6:.1f} Gpairs/s{same}", flush=True)
-    os.environ["PG_KNN_VARIANT"] = "0"
+        best = min(best, a.elapsed_time(b))
+    print(f"{best:.2f} ms  {args.n * args.n / best / 1e6:.1f} Gpairs/s", flush=True)
 
 
 if __name__ == "__main__":

@@ -22,7 +22,6 @@ def main():
     ap.add_argument("--length", type=int, default=256)
     ap.add_argument("--k", type=int, default=16)
     ap.add_argument("--dist", default="uniform")
-    ap.add_argument("--pair", default="0", help=argparse.SUPPRESS)      # instantiations measured in round 2 and removed
     ap.add_argument("--delay", default="0", help=argparse.SUPPRESS)
     ap.add_argument("--band", default="0,24")
     ap.add_argument("--boot", default="8192")
@@ -43,10 +42,10 @@ def main():
     if args.stats:
         os.environ["PG_SYM_STATS"] = "1"
     ranks = list(range(args.world)) if args.rank < 0 else [args.rank]
-    for pair, delay, band, boot, rank in itertools.product(args.pair.split(","), args.delay.split(","), args.band.split(","),
-                                                           args.boot.split(","), ranks):
+    for delay, band, boot, rank in itertools.product(args.delay.split(","), args.band.split(","), args.boot.split(","),
+                                                     ranks):
         args.rank = rank
-        os.environ["PG_SYM_PAIR"], os.environ["PG_SYM_BAND_MB"], os.environ["PG_SYM_BOOT"] = pair, band, boot
+        os.environ["PG_SYM_BAND_MB"], os.environ["PG_SYM_BOOT"] = band, boot
         os.environ["PG_SYM_DELAY"] = delay
         best = None
         for _ in range(args.reps):
@@ -73,7 +72,7 @@ def main():
             eng.time_sweeps(False)
             if best is None or ms < best[0]:
                 best = (ms, sw)
-        print(json.dumps({"n": n, "dist": args.dist, "eps": args.eps, "world": args.world, "rank": args.rank, "pair": pair,
+        print(json.dumps({"n": n, "dist": args.dist, "eps": args.eps, "world": args.world, "rank": args.rank,
                           "delay": delay, "band_mb": band, "boot": boot, "build_ms": round(best[0], 2),
                           "sweeps_ms": [round(v, 2) for v in best[1]],
                           "gpairs_n2": round(n * n / best[0] / 1e6, 1)}), flush=True)
